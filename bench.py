@@ -19,6 +19,11 @@ Timed regions are bracketed by a barrier and a device synchronise on both sides 
 roofline comes from CUDA events recorded on the launching stream inside libvgb200.so.  A multi-rank run checks its own
 result: rank 0 re-processes every rank's batches on its own GPU and compares the raw counters and the calls with what the
 NCCL all-reduce left ("parity_checked"); a mismatch exits non-zero.
+
+`--dump-outputs DIR` writes what the HBM-resident leg (the one `value` is quoted on) left behind after its last step -- per-site
+counters and calls, on a seeded sample of the sites when there are more than DUMP_SITES, and the counters of the timed steps --
+as float32 / float64 .npy files.  Index and reads are generated from fixed seeds, so two builds run with the same arguments on
+the same workload (the line's config.workload) can be compared output for output.
 """
 from __future__ import annotations
 
@@ -46,6 +51,11 @@ READ_SETS = {"s1": (0.005, 0.25), "s2": (0.005, 0.25), "s3": (0.02, 1.0)}
 FALLBACK_MARK = "/tmp/vgb200_bench_workload_fallback"
 KERNEL_SOURCES = ["vargeno_b200/csrc/vgb_geno8.inl", "vargeno_b200/csrc/vgb_geno.cu", "vargeno_b200/csrc/vgb_common.cuh",
                   "vargeno_b200/csrc/vgb_index.cu"]
+# --dump-outputs: at most this many SNP sites are written (a fixed, seeded sample of the GRCh38-shaped list keeps the files near
+# 28 MB); the counters are the ones tests compare with the oracle (timings and chunk bookkeeping left out)
+DUMP_SITES = 1 << 20
+DUMP_COUNTERS = ("reads", "skipped_n", "passes", "placed", "exact_lookups", "nbr_query_lookups", "nbr_scan_reads", "bf_probes",
+                 "lowq_kmers", "events", "pileup_incr", "big_kmers")
 
 
 def rec_bytes(read_len=READ_LEN):
@@ -321,6 +331,7 @@ def run_ours(args):
     time.sleep(0.5)                         # nvidia-smi needs a moment to come up; samples cover both timed legs
     dt, st0, st1 = resident_leg(d_reads, first)
     main = leg_numbers(dt, st0, st1)
+    dump = job_outputs(g, st0, st1) if args.dump_outputs and rank == 0 else None
 
     # ---- kernel durations for the roofline: the same steps with every kernel alone on the GPU ----
     # In production the hand-over kernels of a chunk (a few thousand reads from repeat families, a long dependent chain each) run
@@ -497,6 +508,8 @@ def run_ours(args):
             out["shapes"] = shapes
         if fallback_note:
             out["workload_fallback"] = fallback_note
+        if dump:
+            out["dump_outputs"] = write_outputs(args.dump_outputs, dump)
         emit(out)
     g.dfree(d_reads)
     g.close()
@@ -511,6 +524,28 @@ def host_sample(g, wl, d_buf, n, first_id, sub_rate, lowq_prob):
     from vargeno_b200.tools import device_workloads as dw
     dw.synth_batch(g, wl, d_buf, n, first_id, sub_rate, lowq_prob, LOWQ_CHARS, REC_ID_WIDTH)
     return g.d2h(d_buf, n * rec_bytes())
+
+
+def job_outputs(g, s0, s1):
+    """What a caller of the timed path holds after its last step: per-site ref / alt counters (all-reduced when N > 1) and the
+    calls (GT code, confidence), on all sites or on a sorted sample of DUMP_SITES drawn with a fixed seed (the sample depends
+    only on the site count, so two builds dump the same sites), plus the counters of the K timed steps."""
+    ref_cnt, alt_cnt = g.pileup()
+    gt, conf = g.call()
+    n = ref_cnt.size
+    idx = np.arange(n) if n <= DUMP_SITES else np.sort(np.random.default_rng(0).choice(n, DUMP_SITES, replace=False))
+    return {"site_index": idx.astype(np.float64), "ref_cnt": ref_cnt[idx].astype(np.float32), "alt_cnt": alt_cnt[idx].astype(np.float32),
+            "gt": gt[idx].astype(np.float32), "conf": conf[idx].astype(np.float64),
+            "counters": np.array([s1[k] - s0[k] for k in DUMP_COUNTERS], dtype=np.float64)}
+
+
+def write_outputs(d, arrays):
+    """<d>/<name>.npy per array; returns what the JSON line says about it."""
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), a)
+    return {"dir": d, "files": sorted(name + ".npy" for name in arrays), "sites": int(arrays["site_index"].size),
+            "bytes": int(sum(a.nbytes for a in arrays.values())), "counters": list(DUMP_COUNTERS)}
 
 
 def cpu_port_baseline(index, text, stress_text=None):
@@ -809,7 +844,11 @@ def main():
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--skip-shapes", action="store_true", help="do not run the S3 / S4 legs after the S2 legs")
     ap.add_argument("--skip-roofline-probe", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path computed (site counters, calls, step counters) as DIR/<name>.npy, to compare builds")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the CUDA path computed: it does not apply to --impl reference")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

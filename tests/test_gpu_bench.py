@@ -6,16 +6,18 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def test_bench_line_at_small_scale():
+def test_bench_line_at_small_scale(tmp_path):
+    dump = str(tmp_path / "outputs")
     p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--scale", "0.004", "--steps", "2", "--warmup", "3", "--batch-reads", "20000",
-                        "--cpu-sample", "6000", "--probe-launches", "1", "--clock-hold-s", "0"], stdout=subprocess.PIPE, stderr=subprocess.PIPE,
-                       text=True, timeout=900, cwd=ROOT)
+                        "--cpu-sample", "6000", "--probe-launches", "1", "--clock-hold-s", "0", "--dump-outputs", dump],
+                       stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=900, cwd=ROOT)
     assert p.returncode == 0, p.stderr[-2000:]
     lines = [l for l in p.stdout.splitlines() if l.startswith("{")]
     assert len(lines) == 1, p.stdout[-2000:]
@@ -36,3 +38,13 @@ def test_bench_line_at_small_scale():
     assert c["parity_s3"]["parity_checked"] is True and c["parity_s3"]["reads_compared"] == 1500 and c["parity_s3"]["counters_differing"] == []
     assert d["gpu_launches"] > 0
     assert set(d["shapes"]) == {"s3", "s4"} and d["shapes"]["s3"]["value"] > 0
+    # --dump-outputs: float arrays of what the timed leg computed; the step counters cover exactly the --steps timed steps
+    o = d["dump_outputs"]
+    got = {f[:-4]: np.load(os.path.join(dump, f)) for f in sorted(os.listdir(dump))}
+    assert sorted(got) == ["alt_cnt", "conf", "counters", "gt", "ref_cnt", "site_index"] and o["files"] == sorted(f + ".npy" for f in got)
+    assert all(a.dtype in (np.float32, np.float64) for a in got.values()) and sum(a.nbytes for a in got.values()) <= 64 << 20
+    n = min(d["config"]["snp_sites"], 1 << 20)
+    assert o["sites"] == n and all(got[k].shape == (n,) for k in ("site_index", "ref_cnt", "alt_cnt", "gt", "conf"))
+    counters = dict(zip(o["counters"], got["counters"]))
+    assert counters["reads"] == 2 * 20000 and counters["placed"] > 0
+    assert np.count_nonzero(got["ref_cnt"] + got["alt_cnt"]) > 0 and np.isin(got["gt"], [0, 1, 2, 3]).all()
