@@ -197,7 +197,7 @@ def test_format_violations_are_loud(cache):
 def test_long_reads_and_context_overflow_take_the_deferred_path(cache):
     """Reads of 288+ bases (more than 8 k-mers) and reads with more hit contexts than the group kernels (4 or 8 lanes per read) keep in shared
     memory are handed on: up to 64 contexts per pass to the wide-list instantiation (8 lanes per read), beyond that and beyond 8 k-mers to the
-    warp-per-read kernel; results must not depend on which kernel handled a read."""
+    last stage (32 lanes, one read per warp, contexts spilled to global memory); results must not depend on which kernel handled a read."""
     from vargeno_b200.geno import Genotyper
     from vargeno_b200.tools import synth
     import datasets
@@ -244,28 +244,27 @@ def test_long_reads_and_context_overflow_take_the_deferred_path(cache):
         assert st[k] == ost[k], k
     n_ctx = want["n_ref"].astype(int) + want["n_snp"].astype(int)
     assert int(np.count_nonzero((n_ctx > 24) & (n_ctx <= 64))) > 0, "the set should contain reads for the wide-list kernel (25..64 contexts in a pass)"
-    assert int(n_ctx.max()) > 64, "the set should contain reads beyond the wide list as well (warp-per-read kernel)"
+    assert int(n_ctx.max()) > 64, "the set should contain reads beyond the wide list as well (last stage, spilled contexts)"
     # short reads (<= 8 k-mers) whose RETRY pass overflows the budget: the 4-lane kernel has already run and accounted for their
     # forward pass and hands over only the retry (bit 31 of the deferred-list entry)
     short = np.arange(want.size) >= n_before_retry_set
     n_retry_overflow = int(np.count_nonzero(short & (want["passes"] == 2) & (want["n_ref"].astype(int) + want["n_snp"].astype(int) > 24)))
     assert n_retry_overflow > 0, "the set should contain short reads that overflow in the retry pass"
     o.close()
-    # the warp-per-read kernel alone gives the same answer, and so does the chain without the wide-list kernel
-    for knob, val in (("VGB_GENO_KERNEL", "warp"), ("VGB_NO_WIDE", "1")):
-        os.environ[knob] = val
-        try:
-            with Genotyper(device=0, trace=True, max_chunk_bytes=1 << 20) as g:
-                g.upload_index(ix)
-                g.submit(fq)
-                g.sync()
-                got2 = g.read_results()
-                st2 = g.stats()
-        finally:
-            os.environ.pop(knob, None)
-        assert np.array_equal(got, got2), knob
-        for k in ("reads", "passes", "placed", "exact_lookups", "nbr_query_lookups", "nbr_scan_reads", "events", "pileup_incr", "big_kmers"):
-            assert st2[k] == st[k], (knob, k)
+    # the chain without the wide-list kernel gives the same answer: the 25..64-context reads then go to the last stage as well
+    os.environ["VGB_NO_WIDE"] = "1"
+    try:
+        with Genotyper(device=0, trace=True, max_chunk_bytes=1 << 20) as g:
+            g.upload_index(ix)
+            g.submit(fq)
+            g.sync()
+            got2 = g.read_results()
+            st2 = g.stats()
+    finally:
+        os.environ.pop("VGB_NO_WIDE", None)
+    assert np.array_equal(got, got2)
+    for k in ("reads", "passes", "placed", "exact_lookups", "nbr_query_lookups", "nbr_scan_reads", "events", "pileup_incr", "big_kmers"):
+        assert st2[k] == st[k], k
 
 
 def test_device_read_simulator_matches_numpy(cache):

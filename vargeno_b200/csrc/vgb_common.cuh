@@ -227,11 +227,6 @@ __device__ __forceinline__ void ref_lo_gate_bucket(const DevIndex &ix, uint32_t 
 	s = a.x + cs;
 	e = a.x + ce;
 }
-__device__ __forceinline__ void ref_lo_bucket(const DevIndex &ix, uint32_t lo32, uint32_t &s, uint32_t &e)
-{
-	bool gate;
-	ref_lo_gate_bucket(ix, lo32, gate, s, e);
-}
 // BloomFilter::check_value, value_range 32 (src/generate_bf.h:112-114), through the precomputed gate bit
 __device__ __forceinline__ bool bf_ref(const DevIndex &ix, uint32_t lo32)
 {
@@ -301,15 +296,6 @@ __device__ __forceinline__ bool scan_candidate(uint32_t klo, uint32_t entry32)
 {
 	const uint32_t x = klo ^ entry32;
 	return x == 0u || one_base_slot((uint64_t)x) >= 0;
-}
-// Step s of the reference's strided scan over the SNP block that starts at rank lo (F13): does the entry it examines, rank
-// lo + 11 s, differ from `kmer` in exactly one of the lower 20 bases?  -> that base and the entry's LO40, or -1
-__device__ __forceinline__ int snp_scan_step(const DevIndex &ix, uint32_t lo, uint32_t s, uint64_t kmer, uint64_t &entry_lo40)
-{
-	const uint32_t e32 = ldr(ix.snp_scan + (uint64_t)(lo % SNP_STRIDE) * ix.snp_scan_stride + lo / SNP_STRIDE + s);
-	if (!scan_candidate((uint32_t)kmer, e32)) return -1;
-	entry_lo40 = ldr(&ix.snp[(uint64_t)lo + (uint64_t)SNP_STRIDE * s].key) & 0xFFFFFFFFFFull;
-	return one_base_slot((kmer & 0xFFFFFFFFFFull) ^ entry_lo40);
 }
 // exact membership through the block of the top 30 bits (entry rank inside the HI24 block is not needed there)
 __device__ __forceinline__ int64_t snp_query(const DevIndex &ix, uint64_t kmer, SnpEntry &out)

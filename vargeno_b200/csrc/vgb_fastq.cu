@@ -158,16 +158,9 @@ static cudaError_t launch_fq_index(Chunk &ck, uint64_t nbytes, uint64_t line_cap
 int fastq_index_lines(vgb_ctx *c, Chunk &ck, uint64_t nbytes, cudaStream_t st, int window, uint64_t ov, int last)
 {
 	const uint64_t line_cap = c->max_chunk_bytes / 2 + 16;
-	const int variant = getenv("VGB_FQ_VARIANT") ? atoi(getenv("VGB_FQ_VARIANT")) : 0;   // tuning aid (tools/perf_sweep.py)
 	// measured on B200, 632 MB of FASTQ (profiles/r01_summary.md): 256 x 256 B 0.225 ms, 128 x 256 B 0.235, 512 x 128 B 0.262,
 	// 256 x 128 B 0.267, 128 x 128 B 0.281, 1024 x 64 B 0.293 -- bytes in flight per thread matter more than the tile size
-	cudaError_t e;
-	switch (variant) {
-	case 1: e = launch_fq_index<512, 128>(ck, nbytes, line_cap, st); break;
-	case 2: e = launch_fq_index<256, 512>(ck, nbytes, line_cap, st); break;
-	default: e = launch_fq_index<256, 256>(ck, nbytes, line_cap, st); break;
-	}
-	VGB_CUDA(c, e);
+	VGB_CUDA(c, (launch_fq_index<256, 256>(ck, nbytes, line_cap, st)));
 	k_fq_finish<<<1, 1, 0, st>>>(ck.d_text, nbytes, ck.d_meta + 4, ck.d_meta, ck.d_line_start, line_cap, window, ov, last);
 	c->launches += 2;
 	VGB_CUDA(c, cudaGetLastError());

@@ -24,13 +24,13 @@ struct Chunk {          // one in-flight FASTQ chunk (two slots: copy of chunk i
 	char *h_pinned = nullptr;         // pinned staging buffer handed out by vgb_pinned_buffer
 	uint32_t *d_line_start = nullptr; // [max_lines + 1] byte offset of each line start
 	uint32_t *d_blk_counts = nullptr; // newline count per 4 KiB tile, then its exclusive scan
-	uint32_t *d_defer = nullptr;      // read indices the group kernels hand to the warp-per-read kernel
+	uint32_t *d_defer = nullptr;      // read indices the 4- and 8-lane kernels hand to the wide-list kernel (or the last one)
 	uint32_t *d_defer2 = nullptr;     // read indices the 4-lane kernel hands to the 8-lane kernel
-	uint32_t *d_defer3 = nullptr;     // read indices the wide-list kernel hands to the warp-per-read kernel
+	uint32_t *d_defer3 = nullptr;     // read indices the wide-list kernel hands to the one-warp-per-read kernel
 	uint8_t *d_comp = nullptr;        // BGZF: compressed members of the chunk (allocated at the first vgb_submit_bgzf)
 	BgzfBlock *d_blk = nullptr, *h_blk = nullptr;   // their table, device copy and pinned staging
 	uint32_t blk_cap = 0;
-	uint32_t *d_meta = nullptr;       // [0] n_lines [1] n_reads [2] work counter [3] format error [5] sticky errors [6] deferred reads [7] their work counter [8] framing tile counter [9] reads for the 8-lane kernel [10] their work counter [11] first line of the chunk's own records [12] BGZF member counter [13] reads for the warp kernel [14] their work counter
+	uint32_t *d_meta = nullptr;       // [0] n_lines [1] n_reads [2] work counter [3] format error [5] sticky errors [6] deferred reads [7] their work counter [8] framing tile counter [9] reads for the 8-lane kernel [10] their work counter [11] first line of the chunk's own records [12] BGZF member counter [13] reads for the one-warp-per-read kernel [14] their work counter
 	cudaEvent_t copied = nullptr, done = nullptr, t0 = nullptr, t1 = nullptr, g0 = nullptr;
 	cudaEvent_t g1 = nullptr, h0 = nullptr;   // end of the main kernels on the kernel stream, start of the hand-over kernels on the tail stream
 	bool tail = false;                        // this chunk's hand-over kernels went to the tail stream (`done` is recorded there)
@@ -44,7 +44,7 @@ struct vgb_ctx {
 	int device = 0;
 	int sm_count = 148;
 	cudaStream_t stream = nullptr, copy_stream = nullptr;   // kernels | H2D copies (chunk i+1 is copied under the kernels of chunk i)
-	// The hand-over kernels of a chunk (wide-list stage, warp-per-read kernel: a few thousand reads from repeat families, a long
+	// The hand-over kernels of a chunk (wide-list stage, one-warp-per-read stage: a few thousand reads from repeat families, a long
 	// dependent chain each, the GPU mostly idle) run here, under the framing and the main kernel of the NEXT chunk.  Not in trace mode.
 	cudaStream_t tail_stream = nullptr;
 	bool tail_overlap = false;
@@ -68,16 +68,13 @@ struct vgb_ctx {
 	uint64_t trace_cap = 0, trace_n = 0;
 	uint32_t sticky_format = 0;      // format error bits seen since the last reset
 	bool upload_from_device = false; // vgb_index_upload_device: the index view holds device pointers
-	void *d_spill = nullptr;         // per-warp overflow area for hit contexts
+	void *d_spill = nullptr;         // per-warp overflow area for hit contexts of the last stage
 	uint8_t *d_call_gt = nullptr;    // per-site output staging of vgb_call / vgb_fetch_pileup (allocated once, at first use)
 	double *d_call_conf = nullptr;
 	uint32_t *d_fetch_ref = nullptr, *d_fetch_alt = nullptr;
-	uint32_t geno_grid = 0;
-	// kernel choice of this context (geno_prepare): instantiation + persistent grid per kernel; nothing process-wide
-	void *warp_kernel = nullptr;
-	void *grp_kernel[3][2] = {};     // [0: 4 lanes per read, 1: 8 lanes, 2: 8 lanes with the wide context list][trace]
-	uint32_t grp_grid[3] = {};
-	bool use_quad = true;
+	// kernel choice of this context (geno_prepare): instantiation + persistent grid per stage; nothing process-wide
+	void *grp_kernel[4][2] = {};     // [0: 4 lanes per read, 1: 8 lanes, 2: 8 lanes with the wide context list (nullptr: VGB_NO_WIDE), 3: 32 lanes][trace]
+	uint32_t grp_grid[4] = {};
 	bool inflate_ready = false;       // k_inflate_bgzf: shared-memory attribute set, grid sized
 	uint32_t inflate_grid = 0;
 

@@ -1,7 +1,7 @@
 """Tuning helper: build the S1 workload once, then time the resident-input leg for several library variants
 (environment knobs read by libvgb200.so at context creation / index upload).
 
-    python -m vargeno_b200.tools.perf_sweep VGB_GENO_MINB=4 VGB_GENO_MINB=6 ...   [--scale S] [--batch-reads B] [--steps K]
+    python -m vargeno_b200.tools.perf_sweep "" VGB_SHORTSCAN=0 VGB_SHORTSCAN=1 VGB_NO_TAIL_OVERLAP=1 ...   [--scale S] [--batch-reads B] [--steps K]
 """
 from __future__ import annotations
 

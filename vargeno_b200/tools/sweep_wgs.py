@@ -1,7 +1,7 @@
 """Tuning helper at GRCh38 size: build the S2 index once, then time the resident-input leg on S2 and S3 reads for several
 settings of the VGB_* kernel knobs (re-read by the library at vgb_reset_counts when VGB_RETUNE is set), and the S4 probe sets.
 
-    python -m vargeno_b200.tools.sweep_wgs "" VGB_CARVEOUT=50 VGB_GENO4_MINB=3 ...   [--scale S] [--steps K]
+    python -m vargeno_b200.tools.sweep_wgs "" VGB_SHORTSCAN=1 VGB_NO_WIDE=1 ...   [--scale S] [--steps K]
 (VGB200_LIB=<other build of libvgb200.so> selects a compile-time variant, one process per variant.)
 """
 from __future__ import annotations
