@@ -155,6 +155,16 @@ int  vgb_submit_fastq_device(vgb_ctx *ctx, const char *device_chunk, uint64_t nb
 typedef struct { uint32_t comp_offset, comp_len, out_len; } vgb_bgzf_member;
 int  vgb_submit_bgzf(vgb_ctx *ctx, const void *comp, uint64_t comp_bytes, const vgb_bgzf_member *members, uint32_t n_members,
                      uint64_t overlap_bytes, int last_chunk);
+/* Single-stream gzip input (gzip, pigz, Python's gzip: one member or several back to back, no BGZF index): inflated on the device.
+ * The caller feeds a stream's bytes in order, in pieces of any size up to max_chunk_bytes (host memory; a vgb_pinned_buffer is
+ * copied without staging; the buffer may be reused when the call returns).  first: a new gzip stream starts with this piece (the
+ * last 32 KiB of text of the previous stream stay in front of it, so a record may span two streams, as two files read back to
+ * back); last: the input ends with this piece (a trailing partial record is a format error).  The caller never needs to know block
+ * boundaries or the compression ratio: the library keeps the exact bit cursor, the compressed bytes not consumed yet and the last
+ * 32 KiB of text on the device.  Bytes behind the last member that do not start a gzip member end the input.  A corrupt or
+ * truncated stream, a member whose CRC32 or ISIZE does not match its text, and a single DEFLATE block that needs more than
+ * max_chunk_bytes of input or of text are reported by vgb_sync as VGB_E_FORMAT.  One context inflates a stream. */
+int  vgb_submit_gzip(vgb_ctx *ctx, const void *comp, uint64_t comp_bytes, int first, int last);
 int  vgb_sync(vgb_ctx *ctx);
 int  vgb_reset_counts(vgb_ctx *ctx);              /* zero the pileup counters, statistics and the trace */
 int  vgb_fetch_read_results(vgb_ctx *ctx, vgb_read_result *out, uint64_t cap, uint64_t *n);   /* needs VGB_CFG_TRACE */

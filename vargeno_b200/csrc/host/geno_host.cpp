@@ -521,6 +521,47 @@ int stream_bgzf(const std::vector<vgb_ctx *> &ctxs, const std::vector<MappedFile
 }
 }  // namespace
 
+// ---------------------------------------------------------------------------------------------------------------
+// Single-stream gzip (gzip, pigz, Python's gzip; also BGZF files in a list that is not all BGZF): the files are mapped and fed
+// in pieces through the pinned pair to ONE context (vgb_submit_gzip), which inflates them on the device.  The files are one text
+// stream read back to back: each starts a new gzip stream, and a record may span two of them.  Spreading one gzip stream over
+// several GPUs is not done: with --gpus N the other contexts stay idle.
+// ---------------------------------------------------------------------------------------------------------------
+namespace {
+bool gzip_files(const std::vector<std::string> &paths, std::vector<MappedFile> &files)
+{
+	files.resize(paths.size());
+	for (size_t f = 0; f < paths.size(); f++) {
+		std::string e;
+		if (!files[f].open(paths[f], e) || files[f].size < 2 || files[f].data[0] != 0x1f || files[f].data[1] != 0x8b) return false;
+	}
+	return !files.empty();
+}
+
+int stream_gzip(vgb_ctx *ctx, const std::vector<MappedFile> &files, uint64_t &n_chunks, std::string &err)
+{
+	int slot = 0;
+	n_chunks = 0;
+	for (size_t f = 0; f < files.size(); f++) {
+		for (uint64_t off = 0; off < files[f].size || off == 0;) {
+			char *buf = nullptr;
+			uint64_t cap = 0;
+			int rc = vgb_pinned_buffer(ctx, slot, &buf, &cap);
+			if (rc != VGB_OK) { err = vgb_last_error(ctx); return rc; }
+			const uint64_t n = std::min(cap, files[f].size - off);
+			memcpy(buf, files[f].data + off, n);
+			const bool last = f + 1 == files.size() && off + n == files[f].size;
+			if ((rc = vgb_submit_gzip(ctx, buf, n, off == 0, last)) != VGB_OK) { err = vgb_last_error(ctx); return rc; }
+			off += n;
+			slot ^= 1;
+			n_chunks++;
+			if (n == 0) break;
+		}
+	}
+	return VGB_OK;
+}
+}  // namespace
+
 int stream_fastq(const std::vector<vgb_ctx *> &ctxs, const std::string &path, uint64_t chunk_bytes, uint64_t &n_chunks, std::string &err)
 {
 	std::vector<std::string> paths;
@@ -538,6 +579,11 @@ int stream_fastq(const std::vector<vgb_ctx *> &ctxs, const std::string &path, ui
 		std::vector<BgzfMember> mem;
 		if (!paths.empty() && !getenv("VGB_SEQUENTIAL_READER") && !getenv("VGB_HOST_INFLATE") && bgzf_scan(paths, files, mem))
 			return stream_bgzf(ctxs, files, mem, chunk_bytes, n_chunks, err);
+	}
+	{
+		std::vector<MappedFile> files;
+		if (!paths.empty() && !getenv("VGB_SEQUENTIAL_READER") && !getenv("VGB_HOST_INFLATE") && gzip_files(paths, files))
+			return stream_gzip(ctxs[0], files, n_chunks, err);
 	}
 	return stream_fastq_to(sink, path, chunk_bytes, n_chunks, err);
 }

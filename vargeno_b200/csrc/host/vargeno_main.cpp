@@ -16,6 +16,8 @@ static void print_help()
 	fprintf(stderr, "geno    Perform genotyping (B200)     <index_prefix> <input FASTQ> <input SNPs in VCF> <output file in VCF> "
 	                "[--gpus N] [--chunk-mb M] [--verbose]\n");
 	fprintf(stderr, "        (<input FASTQ>: one file or a comma-separated list read back to back; each plain or gzip)\n");
+	fprintf(stderr, "        (gzip input is inflated on the GPU: BGZF over all GPUs, single-stream gzip on the first GPU only;\n"
+	                "         pipes and lists that mix plain and gzip files are inflated on the host)\n");
 	fprintf(stderr, "filt    Keep the reference-dictionary entries near SNPs   <ref.dict> <snp_locs> <out.dict>   (the reference's hidden `filt`)\n");
 	fprintf(stderr, "index   Build the index (B200)         <input FASTA> <input SNPs in VCF> <index_prefix> [--gpu D] [--no-lite] [--verbose]\n");
 	fprintf(stderr, "        (the same files as the reference's `vargeno index`, byte for byte; --no-lite skips the 2.3 GB .ref.bf.lite.bf that nothing reads)\n");

@@ -21,8 +21,6 @@ int set_err(vgb_ctx *c, int code, const char *fmt, ...)
 	return code;
 }
 
-static void collect_times(vgb_ctx *c, int slot);
-
 }  // namespace vgb
 
 using namespace vgb;
@@ -140,6 +138,7 @@ void vgb_ctx_destroy(vgb_ctx *c)
 		if (k.g1) cudaEventDestroy(k.g1);
 		if (k.h0) cudaEventDestroy(k.h0);
 	}
+	gzip_free(c);
 	cudaFree(c->d_stats); cudaFree(c->d_tables); cudaFree(c->d_trace);
 	for (int i = 0; i < 4; i++) if (c->ev[i]) cudaEventDestroy(c->ev[i]);
 	if (c->stream) cudaStreamDestroy(c->stream);
@@ -193,7 +192,7 @@ int vgb_pinned_buffer(vgb_ctx *c, int slot, char **ptr, uint64_t *cap)
 
 namespace vgb {
 
-static void collect_times(vgb_ctx *c, int slot)
+void collect_times(vgb_ctx *c, int slot)
 {
 	Chunk &k = c->chunk[slot];
 	if (!k.busy) return;
@@ -211,7 +210,7 @@ static void collect_times(vgb_ctx *c, int slot)
 }
 
 // the text of the chunk is (or will be, in stream order) in k.d_text: record framing, then the per-read kernels
-static int process_text(vgb_ctx *c, Chunk &k, uint64_t nbytes, uint64_t first_read_id, int window, uint64_t ov, int last)
+int process_text(vgb_ctx *c, Chunk &k, uint64_t nbytes, uint64_t first_read_id, int window, uint64_t ov, int last)
 {
 	k.tail = false;
 	if (!window) VGB_CUDA(c, cudaEventRecord(k.t0, c->stream));      // BGZF chunks: recorded in front of the inflate kernel, which counts as parsing
@@ -344,6 +343,12 @@ int vgb_submit_bgzf(vgb_ctx *c, const void *comp, uint64_t comp_bytes, const vgb
 	return submit_bgzf(c, (const uint8_t *)comp, comp_bytes, members, n_members, overlap_bytes, last_chunk);
 }
 
+int vgb_submit_gzip(vgb_ctx *c, const void *comp, uint64_t comp_bytes, int first, int last)
+{
+	if (!c || (comp_bytes && !comp)) return c ? set_err(c, VGB_E_ARG, "null argument") : VGB_E_ARG;
+	return submit_gzip(c, (const uint8_t *)comp, comp_bytes, first, last);
+}
+
 int vgb_sync(vgb_ctx *c)
 {
 	if (!c) return VGB_E_ARG;
@@ -363,6 +368,7 @@ int vgb_sync(vgb_ctx *c)
 	VGB_CUDA(c, vgb::copy_sync(c, &st, c->d_stats, sizeof(st), cudaMemcpyDeviceToHost));
 	c->sticky_format |= bits;
 	if (c->sticky_format & 8) return set_err(c, VGB_E_FORMAT, "BGZF input: a gzip member is corrupt or does not inflate to the size its trailer states");
+	if (c->sticky_format & 16) return set_err(c, VGB_E_FORMAT, "gzip input: %s", c->gz.err.c_str());
 	if (c->sticky_format || st.bad_records)
 		return set_err(c, VGB_E_FORMAT, "FASTQ input violates the contract:%s%s%s (%llu bad records)",
 		               (c->sticky_format & 1) ? " truncated record (line count not a multiple of 4);" : "",

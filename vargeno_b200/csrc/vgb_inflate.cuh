@@ -50,10 +50,13 @@ struct InflateTables {
 	uint16_t code[320];                // canonical code of every symbol (table construction)
 	uint8_t lens[320];                 // code lengths: literal/length alphabet first, distance alphabet behind it
 };
-struct alignas(16) InflateWarp {       // what one warp needs in shared memory
-	uint8_t ring[INF_WIN];
+template <typename T>
+struct alignas(16) InflateWarpT {      // what one warp needs in shared memory
+	T ring[INF_WIN];
 	InflateTables t;
 };
+using InflateWarp = InflateWarpT<uint8_t>;     // BGZF members: bytes
+using InflateWarp16 = InflateWarpT<uint16_t>;  // speculative sub-streams of a single gzip stream: bytes and window markers
 
 enum { INF_OK = 0, INF_E_INPUT = 1, INF_E_OUTPUT = 2, INF_E_CODE = 3, INF_E_DIST = 4, INF_E_BTYPE = 5, INF_E_STORED = 6 };
 
@@ -294,21 +297,23 @@ INF_HD uint32_t inf_read_lengths(InflateBits &b, InflateTables &t)
 	return r;
 }
 
-// Ring -> text buffer, bytes [from, to) of the output, by the whole warp.  Byte x of the output sits at ring[(x + a0) % INF_WIN]
-// with a0 = the text buffer's address mod 16, so a 16-byte aligned piece of the text is a 16-byte aligned piece of the ring.
-// Without `all` the copy stops at the last 16-byte boundary of the text; returns the new flushed mark (the same in every lane).
-INF_HD uint32_t inf_flush(const uint8_t *ring, uint8_t *out, uint32_t a0, uint32_t from, uint32_t to, bool all)
+// Ring -> text buffer, symbols [from, to) of the output, by the whole warp.  Symbol x of the output sits at ring[(x + a0) % INF_WIN]
+// with a0 = the text buffer's address mod 16 (in symbols), so a 16-byte aligned piece of the text is a 16-byte aligned piece of the
+// ring.  Without `all` the copy stops at the last 16-byte boundary of the text; returns the new flushed mark (the same in every lane).
+template <typename T>
+INF_HD uint32_t inf_flush(const T *ring, T *out, uint32_t a0, uint32_t from, uint32_t to, bool all)
 {
+	constexpr uint32_t V = 16u / sizeof(T);           // symbols per 16 bytes
 	const uint32_t lane = INF_LANE();
 	const uint32_t M = INF_WIN - 1;
 	uint32_t f = from;
-	const uint32_t head = (16u - ((f + a0) & 15u)) & 15u;
+	const uint32_t head = (V - ((f + a0) & (V - 1u))) & (V - 1u);
 	const uint32_t nh = head < to - f ? head : to - f;
 	for (uint32_t i = lane; i < nh; i += INF_LANES) out[f + i] = ring[(f + i + a0) & M];
 	f += nh;
-	const uint32_t nvec = (to - f) >> 4;
-	for (uint32_t v = lane; v < nvec; v += INF_LANES) INF_COPY16(out + f + 16u * v, ring + ((f + 16u * v + a0) & M));
-	f += 16u * nvec;
+	const uint32_t nvec = (to - f) / V;
+	for (uint32_t v = lane; v < nvec; v += INF_LANES) INF_COPY16(out + f + V * v, ring + ((f + V * v + a0) & M));
+	f += V * nvec;
 	if (all) {
 		for (uint32_t i = lane; i < to - f; i += INF_LANES) out[f + i] = ring[(f + i + a0) & M];
 		f = to;
@@ -317,21 +322,47 @@ INF_HD uint32_t inf_flush(const uint8_t *ring, uint8_t *out, uint32_t a0, uint32
 	return f;
 }
 
+// Speculative decoding (SPEC = true) of a piece of a single gzip stream whose preceding 32 KiB of text are not known yet.  Output
+// symbols are 16-bit: a byte value, or INF_MARK + w for "byte w of the window" (w = 0 is the byte 32 KiB in front of the piece's
+// first symbol, w = 32767 the byte right in front of it).  A match that reaches in front of the piece's first symbol emits markers
+// for the bytes it cannot see, and copying a marker copies the marker.  Bit positions are relative to the first bit of `in`.
+constexpr uint32_t INF_MARK = 256, INF_HIST = 32768;
+struct InflateSpec {
+	uint32_t start_bit;                // in: first block header (0..7: `in` is the byte that holds it)
+	uint32_t stop_bit;                 // in: stop at the first block boundary at or past this bit
+	uint32_t end_bit, end_len;         // out: the last block boundary reached and the symbols in front of it
+	uint32_t final_block;              // out: end_bit is the end of a block with BFINAL set
+};
+
 // One DEFLATE stream [in, in + in_len) -> out[0 .. out_cap).  Executed by a whole warp (every lane calls it with the same
-// arguments); returns the same (status, bytes written) in every lane.
-INF_HD int inflate_block(const uint8_t *in, uint64_t in_len, uint8_t *out, uint32_t out_cap, InflateWarp &ws, uint32_t *out_len)
+// arguments); returns the same (status, symbols written) in every lane.  With SPEC the decoder also stops at sp->stop_bit (INF_OK,
+// final_block 0), and every other return leaves in sp the last block boundary it passed; running out of input there is INF_E_INPUT.
+template <bool SPEC, typename T>
+INF_HD int inflate_block_t(const uint8_t *in, uint64_t in_len, T *out, uint32_t out_cap, InflateWarpT<T> &ws, uint32_t *out_len, InflateSpec *sp)
 {
 	enum { EX_EOB = 1, EX_MATCH = 2, EX_FLUSH = 3, EX_ERR = 4 };
 	const uint32_t lane = INF_LANE();
 	const uint32_t M = INF_WIN - 1;
 	InflateTables &t = ws.t;
-	uint8_t *ring = ws.ring;
-	const uint32_t a0 = (uint32_t)(reinterpret_cast<uintptr_t>(out) & 15u);
+	T *ring = ws.ring;
+	const uint32_t a0 = (uint32_t)(reinterpret_cast<uintptr_t>(out) & 15u) / (uint32_t)sizeof(T);
 	InflateBits b;
 	inf_open(b, in, (uint32_t)(in_len < 0x10000000ull ? in_len : 0x10000000ull));
-	uint32_t pos = 0, flushed = 0;     // bytes produced / bytes of them that are in the text buffer; the same in every lane
+	uint32_t pos = 0, flushed = 0;     // symbols produced / symbols of them that are in the text buffer; the same in every lane
 	int status = INF_OK;
+	uint32_t lb_bit = 0, lb_len = 0, fin = 0;   // SPEC: last block boundary (relative bit, symbols in front of it), BFINAL seen
+	if (SPEC) {
+		if (lane == 0) inf_skip(b, sp->start_bit);
+		lb_bit = sp->start_bit;
+	}
 	for (;;) {
+		if (SPEC) {
+			uint32_t at = 0;
+			if (lane == 0) at = b.bp - b.bp0;
+			at = INF_BCAST(at);
+			lb_bit = at; lb_len = pos;
+			if (at >= sp->stop_bit) break;
+		}
 		// ---- block header (lane 0 reads, everybody learns the type) ----
 		uint32_t hdr = 0;
 		if (lane == 0) { hdr = inf_take(b, 3); if (b.bp > b.end) hdr |= 8u; }
@@ -349,15 +380,15 @@ INF_HD int inflate_block(const uint8_t *in, uint64_t in_len, uint8_t *out, uint3
 				len = w & 0xFFFFu;
 				if ((len ^ 0xFFFFu) != (w >> 16)) bad = 1;
 				src = (b.bp - b.bp0) >> 3;
-				if (b.bp > b.end || (uint64_t)src + len > b.n) bad = 1;
+				if (b.bp > b.end || (uint64_t)src + len > b.n) bad = SPEC && (len ^ 0xFFFFu) == (w >> 16) ? 2 : 1;   // 2: runs past the input
 				else inf_seek(b, src + len);
 			}
 			len = INF_BCAST(len); src = INF_BCAST(src); bad = INF_BCAST(bad);
-			if (bad) { status = INF_E_STORED; break; }
+			if (bad) { status = SPEC && bad == 2 ? INF_E_INPUT : INF_E_STORED; break; }
 			if (pos + len > out_cap) { status = INF_E_OUTPUT; break; }
 			flushed = inf_flush(ring, out, a0, flushed, pos, true);
 			for (uint32_t i = lane; i < len; i += INF_LANES) {
-				const uint8_t v = in[src + i];
+				const T v = in[src + i];
 				out[pos + i] = v;
 				if (len - i <= INF_WIN) ring[(pos + i + a0) & M] = v;
 			}
@@ -398,7 +429,7 @@ INF_HD int inflate_block(const uint8_t *in, uint64_t in_len, uint8_t *out, uint3
 						}
 						uint32_t cl = e & 15u;
 						if (cl && (e & 0x300u) == (INF_K_LIT << 8)) {        // a literal out of the direct table: the common case
-							ring[(pos + a0) & M] = (uint8_t)(e >> 16);
+							ring[(pos + a0) & M] = (T)(e >> 16);
 							pos++;
 							inf_skip(b, cl);
 							continue;
@@ -406,7 +437,7 @@ INF_HD int inflate_block(const uint8_t *in, uint64_t in_len, uint8_t *out, uint3
 						if (cl == 0) { e = inf_slow(b, t.lcount, t.lsym, false); win = inf_peek(b); }
 						const uint32_t kind = (e >> 8) & 3u;
 						if (kind == INF_K_LIT) {
-							ring[(pos + a0) & M] = (uint8_t)(e >> 16);
+							ring[(pos + a0) & M] = (T)(e >> 16);
 							pos++;
 							continue;
 						}
@@ -428,7 +459,7 @@ INF_HD int inflate_block(const uint8_t *in, uint64_t in_len, uint8_t *out, uint3
 						// one test for everything that takes the match away from this lane: the three ways it can be wrong, and "long"
 						if ((((e >> 8) & 3u) != INF_K_BASE) | (mdist > pos) | (pos + mlen > out_cap) | (mlen > INF_SOLO)) {
 							if (((e >> 8) & 3u) != INF_K_BASE) { ex = EX_ERR; err = INF_E_CODE; }
-							else if (mdist > pos) { ex = EX_ERR; err = INF_E_DIST; }
+							else if (mdist > pos && !SPEC) { ex = EX_ERR; err = INF_E_DIST; }   // SPEC: markers, copied by the warp
 							else if (pos + mlen > out_cap) { ex = EX_ERR; err = INF_E_OUTPUT; }
 							else ex = EX_MATCH;
 							break;
@@ -440,12 +471,12 @@ INF_HD int inflate_block(const uint8_t *in, uint64_t in_len, uint8_t *out, uint3
 						if (mdist <= INF_REACH) {
 							const uint32_t sr = (pos + a0 - mdist) & M;
 							if (d + mlen <= INF_WIN && sr + mlen <= INF_WIN) {
-								const uint8_t *sp = ring + sr;
-								uint8_t *dp = ring + d;
+								const T *sp = ring + sr;
+								T *dp = ring + d;
 								if (mdist >= 4) {
 									uint32_t i = 0;
 									for (; i + 4 <= mlen; i += 4) {
-										const uint8_t v0 = sp[i], v1 = sp[i + 1], v2 = sp[i + 2], v3 = sp[i + 3];
+										const T v0 = sp[i], v1 = sp[i + 1], v2 = sp[i + 2], v3 = sp[i + 3];
 										dp[i] = v0; dp[i + 1] = v1; dp[i + 2] = v2; dp[i + 3] = v3;
 									}
 									for (; i < mlen; i++) dp[i] = sp[i];
@@ -456,12 +487,12 @@ INF_HD int inflate_block(const uint8_t *in, uint64_t in_len, uint8_t *out, uint3
 								for (uint32_t i = 0; i < mlen; i++) ring[(d + i) & M] = ring[(sr + i) & M];
 							}
 						} else {
-							const uint8_t *sp = out + (pos - mdist);
+							const T *sp = out + (pos - mdist);
 							if (d + mlen <= INF_WIN) {
-								uint8_t *dp = ring + d;
+								T *dp = ring + d;
 								uint32_t i = 0;
 								for (; i + 4 <= mlen; i += 4) {
-									const uint8_t v0 = INF_LOAD_OUT(sp + i), v1 = INF_LOAD_OUT(sp + i + 1), v2 = INF_LOAD_OUT(sp + i + 2), v3 = INF_LOAD_OUT(sp + i + 3);
+									const T v0 = INF_LOAD_OUT(sp + i), v1 = INF_LOAD_OUT(sp + i + 1), v2 = INF_LOAD_OUT(sp + i + 2), v3 = INF_LOAD_OUT(sp + i + 3);
 									dp[i] = v0; dp[i + 1] = v1; dp[i + 2] = v2; dp[i + 3] = v3;
 								}
 								for (; i < mlen; i++) dp[i] = INF_LOAD_OUT(sp + i);
@@ -483,7 +514,18 @@ INF_HD int inflate_block(const uint8_t *in, uint64_t in_len, uint8_t *out, uint3
 				if (ex == EX_MATCH) {
 					// every byte comes from the part of the output that is already complete (i mod distance): out of the ring, or --
 					// further back than the ring reaches -- out of the text buffer
-					if (mdist <= INF_REACH) {
+					if (SPEC && mdist > pos) {
+						// in front of the piece's first symbol: markers for the window bytes, then the piece's own output
+						for (uint32_t i = lane; i < mlen; i += INF_LANES) {
+							const uint32_t j = mdist >= mlen ? i : i % mdist;
+							const int32_t s = (int32_t)(pos + j) - (int32_t)mdist;
+							T v;
+							if (s < 0) v = (T)(INF_MARK + INF_HIST + s);
+							else if (mdist <= INF_REACH) v = ring[((uint32_t)s + a0) & M];
+							else v = INF_LOAD_OUT(out + s);
+							ring[(pos + i + a0) & M] = v;
+						}
+					} else if (mdist <= INF_REACH) {
 						for (uint32_t i = lane; i < mlen; i += INF_LANES) {
 							const uint32_t j = mdist >= mlen ? i : i % mdist;
 							ring[(pos + i + a0) & M] = ring[(pos - mdist + j + a0) & M];
@@ -498,11 +540,26 @@ INF_HD int inflate_block(const uint8_t *in, uint64_t in_len, uint8_t *out, uint3
 			}
 			if (status != INF_OK) break;
 		} else { status = INF_E_BTYPE; break; }
-		if (last) break;
+		if (last) { if (SPEC) fin = 1; break; }
+	}
+	if (SPEC) {
+		// the end of the last block, or -- for an error or a stop -- the last boundary in front of it
+		uint32_t at = 0, over = 0;
+		if (lane == 0) { at = b.bp - b.bp0; over = b.bp > b.end; }
+		at = INF_BCAST(at); over = INF_BCAST(over);
+		if (status == INF_OK && fin) { lb_bit = at; lb_len = pos; }
+		else if (status != INF_OK && over) status = INF_E_INPUT;   // ran out of input inside a block: not an error of the stream
+		sp->end_bit = lb_bit; sp->end_len = lb_len; sp->final_block = fin;
+		if (status != INF_OK) { flushed = inf_flush(ring, out, a0, flushed, pos < out_cap ? pos : out_cap, true); }
 	}
 	if (status == INF_OK) flushed = inf_flush(ring, out, a0, flushed, pos, true);
 	*out_len = pos;
 	return status;
+}
+
+INF_HD int inflate_block(const uint8_t *in, uint64_t in_len, uint8_t *out, uint32_t out_cap, InflateWarp &ws, uint32_t *out_len)
+{
+	return inflate_block_t<false, uint8_t>(in, in_len, out, out_cap, ws, out_len, nullptr);
 }
 
 }  // namespace vgb

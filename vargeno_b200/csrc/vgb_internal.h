@@ -17,6 +17,29 @@ struct DevStats {   // device-resident counters, one cache line apart from nothi
 	    lowq_kmers, events, pileup_incr, big_kmers, bad_records, overflow_reads, freq_wrap_reads, first_error;
 };
 
+struct GzSub;
+struct GzRound;
+// single gzip stream fed by vgb_submit_gzip (vgb_gzip.cu): compressed bytes not consumed yet, exact bit cursor, last 32 KiB of text
+struct GzStream {
+	uint8_t *d_comp = nullptr;        // compressed bytes [0, avail)
+	uint16_t *d_sym = nullptr;        // speculative output of a round, one slice per sub-stream (also the compaction buffer)
+	uint8_t *d_win = nullptr;         // window in front of each sub-stream of a round (32 KiB each)
+	uint8_t *d_tail = nullptr;        // the last 32 KiB of text (framing overlap and the decode window of the next round)
+	GzSub *d_sub = nullptr;
+	GzRound *d_round = nullptr, *h_round = nullptr;
+	uint64_t *d_off = nullptr;        // text offset of each sub-stream of a round
+	uint64_t *d_member = nullptr, *h_member = nullptr;   // member trailer / header parse result
+	cudaEvent_t copied = nullptr, moved = nullptr;       // H2D copy of the last piece / compaction of the unconsumed bytes
+	uint64_t comp_cap = 0, avail = 0, cur = 0;   // cur: bit cursor (byte aligned outside a member's DEFLATE data)
+	uint32_t max_sub = 0, tail_len = 0, dec_avail = 0;
+	uint64_t member_text = 0, members = 0, repairs = 0, subs = 0;
+	uint32_t member_crc = 0;          // CRC-32 of the member's text so far
+	uint32_t *d_crc = nullptr, *h_crc = nullptr;         // CRC-32 of each GZ_CRC_PIECE bytes of a round's text
+	int state = 0;                    // GZ_S_*
+	bool active = false, failed = false;
+	std::string err;
+};
+
 struct BgzfBlock { uint32_t comp_off, comp_len, out_off, out_len; };   // one gzip member of a chunk: DEFLATE payload in the compressed buffer -> place in the text
 
 struct Chunk {          // one in-flight FASTQ chunk (two slots: copy of chunk i+1 overlaps the kernels of chunk i)
@@ -77,6 +100,7 @@ struct vgb_ctx {
 	uint32_t grp_grid[4] = {};
 	bool inflate_ready = false;       // k_inflate_bgzf: shared-memory attribute set, grid sized
 	uint32_t inflate_grid = 0;
+	vgb::GzStream gz;                 // vgb_submit_gzip
 
 	// host-side statistics
 	uint64_t chunks = 0, chunk_bytes = 0, launches = 0;
@@ -133,6 +157,12 @@ int index_upload(vgb_ctx *c, const vgb_index_view *v);
 // vgb_fastq.cu
 int fastq_index_lines(vgb_ctx *c, Chunk &ck, uint64_t nbytes, cudaStream_t st, int window = 0, uint64_t ov = 0, int last = 0);
 int bgzf_inflate(vgb_ctx *c, Chunk &ck, const uint8_t *d_comp, const BgzfBlock *d_blk, uint32_t n_blk, cudaStream_t st);
+// vgb_gzip.cu
+int submit_gzip(vgb_ctx *c, const uint8_t *comp, uint64_t comp_bytes, int first, int last);
+void gzip_free(vgb_ctx *c);
+// vgb_api.cu
+int process_text(vgb_ctx *c, Chunk &k, uint64_t nbytes, uint64_t first_read_id, int window, uint64_t ov, int last);
+void collect_times(vgb_ctx *c, int slot);
 // vgb_geno.cu
 int geno_launch(vgb_ctx *c, Chunk &ck, uint64_t nbytes, uint64_t first_read_id);
 int geno_prepare(vgb_ctx *c);

@@ -156,6 +156,19 @@ class Genotyper:
             self.submit_bgzf(comp, tab, ov, k + 1 == len(plan))
         return len(plan)
 
+    def submit_gzip(self, buf, piece_bytes: int, first: bool = True, last: bool = True) -> int:
+        """A single-stream gzip image (bytes or uint8 array: one or more gzip members) through vgb_submit_gzip in pieces of
+        `piece_bytes` compressed bytes; `first` / `last` mark the first and the last piece as a new stream and the end of the input.
+        Returns the number of calls."""
+        a = np.frombuffer(buf, dtype=np.uint8) if not isinstance(buf, np.ndarray) else np.ascontiguousarray(buf, dtype=np.uint8)
+        step = max(1, min(int(piece_bytes), self.max_chunk_bytes))
+        starts = list(range(0, a.size, step)) or [0]
+        for i, s in enumerate(starts):
+            piece = np.ascontiguousarray(a[s:s + step])
+            self._ck(self.L.vgb_submit_gzip(self.h, _lib.ptr(piece), piece.size, 1 if first and i == 0 else 0,
+                                            1 if last and i + 1 == len(starts) else 0))
+        return len(starts)
+
     def submit_device(self, dptr: int, nbytes: int, first_read_id: int = 0) -> None:
         self._ck(self.L.vgb_submit_fastq_device(self.h, C.c_void_p(dptr), nbytes, first_read_id))
 

@@ -5,7 +5,8 @@ read loop as the program reports it (index load excluded, reported separately), 
 
 Everything is made on this box: the S1 index (device builder -> the five files), the reads (device generator -> a file in
 tmpfs, i.e. the page-cache case a warm run sees), the BGZF copy (multi-process zlib level 1, like `bgzip -@`), and a
-single-stream gzip copy of the first 2 GB (the sequential zlib path).  Prints one JSON object per run."""
+single-stream `gzip -1` copy of the first 2 GB, run inflated on the device (vgb_submit_gzip, first GPU only) and, for comparison,
+through host zlib (VGB_HOST_INFLATE=1).  Prints one JSON object per run."""
 from __future__ import annotations
 
 import argparse
@@ -60,7 +61,7 @@ def main():
     bgz = fq + ".bgzf.gz"
     bgzf.compress_file(fq, bgz, procs=max(1, (os.cpu_count() or 2) - 1))
     print(json.dumps({"section": "bgzf written", "bytes": os.path.getsize(bgz), "ratio": size / os.path.getsize(bgz), "seconds": round(time.time() - t0, 1)}), flush=True)
-    gz = None
+    gz, n_small = None, 0
     if not args.skip_gzip:
         gz = fq + ".single.gz"
         n_small = min(size, (2_000_000_000 // rb) * rb)
@@ -102,7 +103,12 @@ def main():
         if gpus == 1:
             run("BGZF, inflated on the host by zlib (sequential reader)", bgz, gpus, args.reads, {"VGB_HOST_INFLATE": "1"}) if size <= 8_000_000_000 else None
             if gz:
-                run("single-stream gzip, first 2 GB (host zlib)", gz, gpus, 0)
+                d = run("single-stream gzip, first 2 GB, inflated on the device", gz, gpus, 0)
+                h = run("single-stream gzip, first 2 GB, inflated on the host by zlib", gz, gpus, 0, {"VGB_HOST_INFLATE": "1"})
+                chk = {"section": "check", "gpus": gpus, "gzip_device_vcf_identical_to_host_zlib": d is not None and d == h}
+                if n_small == size:
+                    chk["gzip_device_vcf_identical_to_plain"] = d is not None and d == a
+                print(json.dumps(chk), flush=True)
     shutil.rmtree(args.dir, ignore_errors=True)
 
 

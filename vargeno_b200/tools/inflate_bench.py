@@ -1,8 +1,10 @@
-"""Device-side BGZF inflate (k_inflate_bgzf) measured alone: S1-like FASTQ text made on the device, written as BGZF by zlib at
-two levels, pushed through vgb_submit_bgzf from pinned memory in chunks; prints the rate at which text comes out of the inflate +
-framing kernels (vgb_stats.gpu_ms_parse: CUDA events around both) and the wall-clock rate of the whole submit loop.
+"""Device-side inflate measured alone: S1-like FASTQ text made on the device and compressed by zlib at two levels, either as BGZF
+pushed through vgb_submit_bgzf (k_inflate_bgzf), or (--mode gzip) as one single gzip stream pushed through vgb_submit_gzip in
+pieces (the sub-stream pipeline of csrc/vgb_gzip.cu).  Prints the rate at which text comes out of the inflate + framing kernels
+(vgb_stats.gpu_ms_parse: CUDA events around both) and the wall-clock rate of the whole submit loop.  --profile adds one
+repetition under torch.profiler and prints the CUDA time of each kernel (the window chain's share of a round is read there).
 
-    python -m vargeno_b200.tools.inflate_bench [--reads 4000000] [--chunk-mb 256] [--levels 1,6]
+    python -m vargeno_b200.tools.inflate_bench [--mode bgzf|gzip] [--reads 4000000] [--chunk-mb 256] [--levels 1,6] [--profile]
 """
 from __future__ import annotations
 
@@ -28,6 +30,9 @@ def main():
     ap.add_argument("--chunk-mb", type=int, default=256, help="inflated bytes per vgb_submit_bgzf call")
     ap.add_argument("--levels", default="1,6")
     ap.add_argument("--repeats", type=int, default=3)
+    ap.add_argument("--mode", choices=("bgzf", "gzip"), default="bgzf")
+    ap.add_argument("--piece-mb", type=int, default=64, help="--mode gzip: compressed bytes per vgb_submit_gzip call")
+    ap.add_argument("--profile", action="store_true")
     args = ap.parse_args()
     sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
     import torch
@@ -45,6 +50,10 @@ def main():
         dw.synth_batch(g, wl, d, args.reads, 0, 0.005, 0.25, bench.LOWQ_CHARS, bench.REC_ID_WIDTH)
         text = g.d2h(d, args.reads * rb).tobytes()
         g.dfree(d)
+        if args.mode == "gzip":
+            for level in (int(x) for x in args.levels.split(",")):
+                _gzip_mode(g, text, level, args)
+            return
         for level in (int(x) for x in args.levels.split(",")):
             t0 = time.time()
             span = 65280 * 256
@@ -76,6 +85,48 @@ def main():
                               "chunks": len(chunks), "compress_s": round(t_comp, 1), "inflate_plus_framing_ms": best[0], "geno_ms": best[2],
                               "inflate_text_gb_per_s": len(text) / (best[0] * 1e-3) / 1e9, "wall_s": best[1],
                               "wall_text_gb_per_s": len(text) / best[1] / 1e9, "wall_reads_per_s": args.reads / best[1]}), flush=True)
+
+
+def _gzip_mode(g, text, level, args):
+    import subprocess
+
+    import torch
+    t0 = time.time()
+    comp = subprocess.run(["gzip", "-%d" % level, "-c"], input=text, stdout=subprocess.PIPE, check=True).stdout
+    t_comp = time.time() - t0
+    piece = min(args.piece_mb << 20, g.max_chunk_bytes)
+    pin = torch.empty(len(comp), dtype=torch.uint8, pin_memory=True).numpy()
+    pin[:] = np.frombuffer(comp, dtype=np.uint8)
+    n_reads = text.count(b"\n") // 4
+    best = None
+    for rep in range(args.repeats + 1):
+        g.reset()
+        t0 = time.perf_counter()
+        calls = g.submit_gzip(pin, piece)
+        g.sync()
+        dt = time.perf_counter() - t0
+        s1 = g.stats()
+        assert s1["reads"] == n_reads, (s1["reads"], n_reads)
+        if rep and (best is None or s1["gpu_ms_parse"] < best[0]):
+            best = (s1["gpu_ms_parse"], dt, s1["gpu_ms_geno"])
+    rec = {"mode": "gzip", "gzip_level": level, "text_bytes": len(text), "gzip_bytes": len(comp), "ratio": len(text) / len(comp), "calls": calls,
+           "compress_s": round(t_comp, 1), "inflate_plus_framing_ms": best[0], "geno_ms": best[2],
+           "inflate_text_gb_per_s": len(text) / (best[0] * 1e-3) / 1e9, "wall_s": best[1], "wall_text_gb_per_s": len(text) / best[1] / 1e9,
+           "wall_reads_per_s": n_reads / best[1]}
+    if args.profile:
+        from torch.profiler import ProfilerActivity, profile
+        g.reset()
+        with profile(activities=[ProfilerActivity.CUDA]) as prof:
+            g.submit_gzip(pin, piece)
+            g.sync()
+        ker = {}
+        for e in prof.events():
+            if e.device_type.name == "CUDA":
+                ker[e.name] = ker.get(e.name, 0.0) + e.device_time / 1e3
+        gz = {k: v for k, v in ker.items() if "k_gz_" in k}
+        rec["kernel_ms"] = {k.split("(")[0]: round(v, 3) for k, v in sorted(ker.items(), key=lambda x: -x[1])[:12]}
+        rec["window_chain_share_of_gzip_kernels"] = sum(v for k, v in gz.items() if "k_gz_window" in k) / max(1e-9, sum(gz.values()))
+    print(json.dumps(rec), flush=True)
 
 
 if __name__ == "__main__":
