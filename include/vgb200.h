@@ -165,6 +165,20 @@ int  vgb_submit_bgzf(vgb_ctx *ctx, const void *comp, uint64_t comp_bytes, const 
  * truncated stream, a member whose CRC32 or ISIZE does not match its text, and a single DEFLATE block that needs more than
  * max_chunk_bytes of input or of text are reported by vgb_sync as VGB_E_FORMAT.  One context inflates a stream. */
 int  vgb_submit_gzip(vgb_ctx *ctx, const void *comp, uint64_t comp_bytes, int first, int last);
+/* BAM input (unaligned or aligned BAM): the reads are the FASTQ records `samtools fastq` writes with its default settings, in file
+ * order -- secondary and supplementary records (flag 0x900) and records without bases are skipped, a record with flag 0x10 is
+ * turned back to the sequenced orientation, bases are =ACMGRSVTWYHKDBN (IUPAC codes other than N stay format errors), quality is
+ * qual + 33, or 1 for a record stored without quality.  A call takes whole BGZF members of one BAM file, in file order (as for
+ * vgb_submit_bgzf: `comp` holds them back to back, members[i] locates the DEFLATE payload of member i and gives its ISIZE), with
+ * an ISIZE sum of at most max_chunk_bytes; max_chunk_bytes must be at most 1 GiB.  first: a new file starts with this call (its
+ * header comes first); last: the file ends with it.  A context takes several files one after the other.  The members are inflated
+ * and the records framed and converted on the device; the bytes a call does not consume (a header not complete yet, the record cut
+ * by the call's end) stay on the device in front of the next call's.  The host reads back a small summary per call (where the
+ * records end, record and text totals), so a call returns once its work is queued behind the previous call's per-read kernels.
+ * Bad magic, a header larger than max_chunk_bytes / 2, a record that fails the record check or is larger than 1 MiB, a record
+ * with more than 1022 bases and a file that ends inside its header or a record are reported by vgb_sync as VGB_E_FORMAT.  CRC32
+ * of the members is not verified. */
+int  vgb_submit_bam(vgb_ctx *ctx, const void *comp, uint64_t comp_bytes, const vgb_bgzf_member *members, uint32_t n_members, int first, int last);
 int  vgb_sync(vgb_ctx *ctx);
 int  vgb_reset_counts(vgb_ctx *ctx);              /* zero the pileup counters, statistics and the trace */
 int  vgb_fetch_read_results(vgb_ctx *ctx, vgb_read_result *out, uint64_t cap, uint64_t *n);   /* needs VGB_CFG_TRACE */

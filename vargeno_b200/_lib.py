@@ -52,7 +52,7 @@ SYMBOLS = ["vgb_abi_version", "vgb_ctx_create", "vgb_ctx_destroy", "vgb_last_err
            "vgb_synth_reads_device", "vgb_device_alloc", "vgb_device_free", "vgb_memcpy_d2h", "vgb_memcpy_h2d",
            "vgb_build_index_device", "vgb_free_index_device", "vgb_index_upload_device", "vgb_synth_genome_device",
            "vgb_memcpy_d2d", "vgb_memset_device", "vgb_comm_init", "vgb_build_ref_lite_bf_device", "vgb_build_snp_bf_ucsc_device", "vgb_submit_bgzf",
-           "vgb_submit_gzip"]
+           "vgb_submit_gzip", "vgb_submit_bam"]
 
 _lib = None
 
@@ -104,6 +104,7 @@ def load():
         "vgb_build_snp_bf_ucsc_device": (i32, [vp, vp, vp, vp, u64, C.POINTER(vp), C.POINTER(u64), C.POINTER(u64)]),
         "vgb_submit_bgzf": (i32, [vp, vp, u64, vp, u32, u64, i32]),
         "vgb_submit_gzip": (i32, [vp, vp, u64, i32, i32]),
+        "vgb_submit_bam": (i32, [vp, vp, u64, vp, u32, i32, i32]),
         "vgb_build_ref_lite_bf_device": (i32, [vp, vp, vp, vp, u32, C.POINTER(vp), C.POINTER(u64), C.POINTER(u64)]),
     }
     for name in SYMBOLS:

@@ -562,6 +562,102 @@ int stream_gzip(vgb_ctx *ctx, const std::vector<MappedFile> &files, uint64_t &n_
 }
 }  // namespace
 
+// ---------------------------------------------------------------------------------------------------------------
+// BAM (unaligned or aligned): BGZF whose first member inflates to "BAM\1".  Each file goes to one context, in calls of whole members
+// (vgb_submit_bam), which inflates them and turns the records into FASTQ text on the device.  The files of a list are handed out
+// largest first, each to the context with the fewest bytes so far, so --gpus N uses every GPU once there are N files.
+// VGB_HOST_INFLATE and VGB_SEQUENTIAL_READER do not apply.
+// ---------------------------------------------------------------------------------------------------------------
+namespace {
+bool is_bam(const std::string &path)
+{
+	MappedFile f;
+	std::string e;
+	if (!f.open(path, e) || f.size < 28) return false;
+	const uint8_t *d = f.data;
+	if (d[0] != 0x1f || d[1] != 0x8b || d[2] != 8 || !(d[3] & 4)) return false;
+	const uint32_t xlen = d[10] | (d[11] << 8);
+	if (12 + xlen > f.size) return false;
+	uint32_t bsize = 0;
+	for (uint32_t x = 0; x + 6 <= xlen;) {
+		const uint8_t *sf = d + 12 + x;
+		const uint32_t slen = sf[2] | (sf[3] << 8);
+		if (sf[0] == 'B' && sf[1] == 'C' && slen == 2) bsize = (sf[4] | (sf[5] << 8)) + 1u;
+		x += 4 + slen;
+	}
+	if (bsize < 12 + xlen + 8 || bsize > f.size) return false;
+	// the first member, inflated with zlib (at most 64 KiB)
+	std::vector<unsigned char> out(65536);
+	z_stream zs{};
+	if (inflateInit2(&zs, -15) != Z_OK) return false;
+	zs.next_in = const_cast<Bytef *>(d + 12 + xlen);
+	zs.avail_in = bsize - (12 + xlen) - 8;
+	zs.next_out = out.data();
+	zs.avail_out = (uInt)out.size();
+	inflate(&zs, Z_FINISH);
+	const uint64_t got = out.size() - zs.avail_out;
+	inflateEnd(&zs);
+	return got >= 4 && !memcmp(out.data(), "BAM\1", 4);
+}
+
+int stream_bam(const std::vector<vgb_ctx *> &ctxs, const std::vector<MappedFile> &files, const std::vector<BgzfMember> &mem, uint64_t chunk_bytes,
+               uint64_t &n_chunks, std::string &err)
+{
+	std::vector<std::vector<size_t>> by_file(files.size());
+	for (size_t i = 0; i < mem.size(); i++) by_file[mem[i].file].push_back(i);
+	std::vector<size_t> order(files.size());
+	for (size_t f = 0; f < order.size(); f++) order[f] = f;
+	std::stable_sort(order.begin(), order.end(), [&](size_t a, size_t b) { return files[a].size > files[b].size; });
+	std::vector<std::vector<size_t>> mine(ctxs.size());
+	std::vector<uint64_t> load(ctxs.size(), 0);
+	for (size_t f : order) {
+		const size_t g = (size_t)(std::min_element(load.begin(), load.end()) - load.begin());
+		mine[g].push_back(f);
+		load[g] += files[f].size;
+	}
+	std::atomic<uint64_t> calls(0);
+	std::vector<std::string> errs(ctxs.size());
+	std::vector<int> rcs(ctxs.size(), VGB_OK);
+	auto feeder = [&](size_t g) {
+		vgb_ctx *ctx = ctxs[g];
+		int slot = 0;
+		std::vector<vgb_bgzf_member> tab;
+		for (size_t f : mine[g]) {
+			const std::vector<size_t> &ms = by_file[f];
+			size_t i = 0;
+			do {
+				char *buf = nullptr;
+				uint64_t cap = 0;
+				if ((rcs[g] = vgb_pinned_buffer(ctx, slot, &buf, &cap)) != VGB_OK) { errs[g] = vgb_last_error(ctx); return; }
+				const size_t i0 = i;
+				uint64_t out = 0, at = 0;
+				tab.clear();
+				while (i < ms.size() && out + mem[ms[i]].isize <= std::min(cap, chunk_bytes) && at + mem[ms[i]].size <= cap) {
+					const BgzfMember &m = mem[ms[i]];
+					memcpy(buf + at, files[f].data + m.off, m.size);
+					tab.push_back(vgb_bgzf_member{ (uint32_t)(at + m.payload_off), m.payload_len, m.isize });
+					out += m.isize;
+					at += m.size;
+					i++;
+				}
+				if ((rcs[g] = vgb_submit_bam(ctx, buf, at, tab.data(), (uint32_t)tab.size(), i0 == 0, i == ms.size())) != VGB_OK) {
+					errs[g] = vgb_last_error(ctx);
+					return;
+				}
+				calls++;
+				slot ^= 1;
+			} while (i < ms.size());
+		}
+	};
+	std::vector<std::thread> th;
+	for (size_t g = 0; g < ctxs.size(); g++) th.emplace_back(feeder, g);
+	for (auto &t : th) t.join();
+	n_chunks = calls.load();
+	for (size_t g = 0; g < ctxs.size(); g++) if (rcs[g] != VGB_OK) { err = errs[g]; return rcs[g]; }
+	return VGB_OK;
+}
+}  // namespace
+
 int stream_fastq(const std::vector<vgb_ctx *> &ctxs, const std::string &path, uint64_t chunk_bytes, uint64_t &n_chunks, std::string &err)
 {
 	std::vector<std::string> paths;
@@ -574,6 +670,17 @@ int stream_fastq(const std::vector<vgb_ctx *> &ctxs, const std::string &path, ui
 	GpuSink sink(ctxs);
 	if (!paths.empty() && !getenv("VGB_SEQUENTIAL_READER") && plain.open(paths) && plain.total() > 0)
 		return stream_plain_parallel(sink, ctxs.size(), plain, chunk_bytes, n_chunks, err);
+	{
+		size_t n_bam = 0;
+		for (const std::string &p : paths) n_bam += is_bam(p);
+		if (n_bam && n_bam < paths.size()) { err = "the input list mixes BAM and non-BAM files: give BAM files only or FASTQ files only"; return VGB_E_ARG; }
+		if (n_bam) {
+			std::vector<MappedFile> files;
+			std::vector<BgzfMember> mem;
+			if (!bgzf_scan(paths, files, mem)) { err = "a BAM file is not well-formed BGZF"; return VGB_E_FORMAT; }
+			return stream_bam(ctxs, files, mem, chunk_bytes, n_chunks, err);
+		}
+	}
 	{
 		std::vector<MappedFile> files;
 		std::vector<BgzfMember> mem;

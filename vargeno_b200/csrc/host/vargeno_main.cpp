@@ -15,9 +15,12 @@ static void print_help()
 	fprintf(stderr, "------  -----------                   ----------\n");
 	fprintf(stderr, "geno    Perform genotyping (B200)     <index_prefix> <input FASTQ> <input SNPs in VCF> <output file in VCF> "
 	                "[--gpus N] [--chunk-mb M] [--verbose]\n");
-	fprintf(stderr, "        (<input FASTQ>: one file or a comma-separated list read back to back; each plain or gzip)\n");
+	fprintf(stderr, "        (<input FASTQ>: one file or a comma-separated list read back to back; each plain or gzip; or BAM files only)\n");
 	fprintf(stderr, "        (gzip input is inflated on the GPU: BGZF over all GPUs, single-stream gzip on the first GPU only;\n"
 	                "         pipes and lists that mix plain and gzip files are inflated on the host)\n");
+	fprintf(stderr, "        (BAM, unaligned or aligned: the reads `samtools fastq` gives, inflated and converted on the GPU; each file\n"
+	                "         on one GPU, largest first; a list may not mix BAM and other files; VGB_HOST_INFLATE and\n"
+	                "         VGB_SEQUENTIAL_READER do not apply)\n");
 	fprintf(stderr, "filt    Keep the reference-dictionary entries near SNPs   <ref.dict> <snp_locs> <out.dict>   (the reference's hidden `filt`)\n");
 	fprintf(stderr, "index   Build the index (B200)         <input FASTA> <input SNPs in VCF> <index_prefix> [--gpu D] [--no-lite] [--verbose]\n");
 	fprintf(stderr, "        (the same files as the reference's `vargeno index`, byte for byte; --no-lite skips the 2.3 GB .ref.bf.lite.bf that nothing reads)\n");

@@ -139,6 +139,7 @@ void vgb_ctx_destroy(vgb_ctx *c)
 		if (k.h0) cudaEventDestroy(k.h0);
 	}
 	gzip_free(c);
+	bam_free(c);
 	cudaFree(c->d_stats); cudaFree(c->d_tables); cudaFree(c->d_trace);
 	for (int i = 0; i < 4; i++) if (c->ev[i]) cudaEventDestroy(c->ev[i]);
 	if (c->stream) cudaStreamDestroy(c->stream);
@@ -277,6 +278,41 @@ static int submit_common(vgb_ctx *c, const char *host_chunk, const char *device_
 	return rc;
 }
 
+// the compressed members of a BGZF call into slot k's buffers (copy stream; the kernel stream waits for it) and their table; *out =
+// the sum of their ISIZEs.  Called with the slot free (collect_times).
+int bgzf_stage(vgb_ctx *c, Chunk &k, int slot, const uint8_t *comp, uint64_t comp_bytes, const vgb_bgzf_member *mem, uint32_t n_mem, uint64_t *out)
+{
+	*out = 0;
+	if (n_mem == 0) return VGB_OK;
+	if (!k.d_comp) VGB_CUDA(c, cudaMalloc((void **)&k.d_comp, c->max_chunk_bytes + 64));
+	if (k.blk_cap < n_mem) {
+		const uint32_t cap = std::max<uint32_t>(n_mem, 2 * k.blk_cap + 1024);
+		if (k.d_blk) cudaFree(k.d_blk);
+		if (k.h_blk) cudaFreeHost(k.h_blk);
+		k.d_blk = nullptr; k.h_blk = nullptr; k.blk_cap = 0;
+		VGB_CUDA(c, cudaMalloc((void **)&k.d_blk, (size_t)cap * sizeof(BgzfBlock)));
+		VGB_CUDA(c, cudaMallocHost((void **)&k.h_blk, (size_t)cap * sizeof(BgzfBlock)));
+		k.blk_cap = cap;
+	}
+	uint64_t o = 0;
+	for (uint32_t i = 0; i < n_mem; i++) {
+		if ((uint64_t)mem[i].comp_offset + mem[i].comp_len > comp_bytes || mem[i].out_len > 65536)
+			return set_err(c, VGB_E_ARG, "BGZF member %u lies outside the chunk or claims more than 64 KiB", i);
+		k.h_blk[i] = BgzfBlock{ mem[i].comp_offset, mem[i].comp_len, (uint32_t)o, mem[i].out_len };
+		o += mem[i].out_len;
+	}
+	if (o > c->max_chunk_bytes) return set_err(c, VGB_E_ARG, "chunk inflates to %llu bytes, more than max_chunk_bytes", (unsigned long long)o);
+	VGB_CUDA(c, cudaMemcpyAsync(k.d_comp, comp, comp_bytes, cudaMemcpyHostToDevice, c->copy_stream));
+	VGB_CUDA(c, cudaMemcpyAsync(k.d_blk, k.h_blk, (size_t)n_mem * sizeof(BgzfBlock), cudaMemcpyHostToDevice, c->copy_stream));
+	VGB_CUDA(c, cudaEventRecord(k.copied, c->copy_stream));
+	VGB_CUDA(c, cudaStreamWaitEvent(c->stream, k.copied, 0));
+	const char *hc = (const char *)comp;
+	auto in_pinned = [&](const Chunk &q) { return q.h_pinned && hc >= q.h_pinned && hc < q.h_pinned + c->max_chunk_bytes; };
+	if (!in_pinned(k) && !in_pinned(c->chunk[slot ^ 1])) VGB_CUDA(c, cudaEventSynchronize(k.copied));
+	*out = o;
+	return VGB_OK;
+}
+
 // BGZF chunk: compressed members over PCIe, inflated on the device straight into the chunk's text buffer
 static int submit_bgzf(vgb_ctx *c, const uint8_t *comp, uint64_t comp_bytes, const vgb_bgzf_member *mem, uint32_t n_mem, uint64_t ov, int last)
 {
@@ -288,35 +324,13 @@ static int submit_bgzf(vgb_ctx *c, const uint8_t *comp, uint64_t comp_bytes, con
 	c->next_slot ^= 1;
 	Chunk &k = c->chunk[slot];
 	collect_times(c, slot);
-	if (!k.d_comp) VGB_CUDA(c, cudaMalloc((void **)&k.d_comp, c->max_chunk_bytes + 64));
-	if (k.blk_cap < n_mem) {
-		const uint32_t cap = std::max<uint32_t>(n_mem, 2 * k.blk_cap + 1024);
-		if (k.d_blk) cudaFree(k.d_blk);
-		if (k.h_blk) cudaFreeHost(k.h_blk);
-		k.d_blk = nullptr; k.h_blk = nullptr; k.blk_cap = 0;
-		VGB_CUDA(c, cudaMalloc((void **)&k.d_blk, (size_t)cap * sizeof(BgzfBlock)));
-		VGB_CUDA(c, cudaMallocHost((void **)&k.h_blk, (size_t)cap * sizeof(BgzfBlock)));
-		k.blk_cap = cap;
-	}
 	uint64_t out = 0;
-	for (uint32_t i = 0; i < n_mem; i++) {
-		if ((uint64_t)mem[i].comp_offset + mem[i].comp_len > comp_bytes || mem[i].out_len > 65536)
-			return set_err(c, VGB_E_ARG, "BGZF member %u lies outside the chunk or claims more than 64 KiB", i);
-		k.h_blk[i] = BgzfBlock{ mem[i].comp_offset, mem[i].comp_len, (uint32_t)out, mem[i].out_len };
-		out += mem[i].out_len;
-	}
-	if (out > c->max_chunk_bytes) return set_err(c, VGB_E_ARG, "chunk inflates to %llu bytes, more than max_chunk_bytes", (unsigned long long)out);
+	const int rs = bgzf_stage(c, k, slot, comp, comp_bytes, mem, n_mem, &out);
+	if (rs != VGB_OK) return rs;
 	if (ov > out) return set_err(c, VGB_E_ARG, "overlap larger than the chunk");
-	VGB_CUDA(c, cudaMemcpyAsync(k.d_comp, comp, comp_bytes, cudaMemcpyHostToDevice, c->copy_stream));
-	VGB_CUDA(c, cudaMemcpyAsync(k.d_blk, k.h_blk, (size_t)n_mem * sizeof(BgzfBlock), cudaMemcpyHostToDevice, c->copy_stream));
-	VGB_CUDA(c, cudaEventRecord(k.copied, c->copy_stream));
-	VGB_CUDA(c, cudaStreamWaitEvent(c->stream, k.copied, 0));
-	const char *hc = (const char *)comp;
-	auto in_pinned = [&](const Chunk &q) { return q.h_pinned && hc >= q.h_pinned && hc < q.h_pinned + c->max_chunk_bytes; };
-	if (!in_pinned(k) && !in_pinned(c->chunk[slot ^ 1])) VGB_CUDA(c, cudaEventSynchronize(k.copied));
 	if (out == 0) { cudaEventRecord(k.done, c->stream); k.busy = true; return VGB_OK; }
 	VGB_CUDA(c, cudaEventRecord(k.t0, c->stream));
-	int rc = bgzf_inflate(c, k, k.d_comp, k.d_blk, n_mem, c->stream);
+	int rc = bgzf_inflate(c, k, k.d_comp, k.d_blk, n_mem, c->stream, reinterpret_cast<uint8_t *>(k.d_text));
 	if (rc != VGB_OK) return rc;
 	return process_text(c, k, out, 0, 1, ov, last);
 }
@@ -349,6 +363,13 @@ int vgb_submit_gzip(vgb_ctx *c, const void *comp, uint64_t comp_bytes, int first
 	return submit_gzip(c, (const uint8_t *)comp, comp_bytes, first, last);
 }
 
+int vgb_submit_bam(vgb_ctx *c, const void *comp, uint64_t comp_bytes, const vgb_bgzf_member *members, uint32_t n_members, int first, int last)
+{
+	if (!c || (n_members && (!comp || !members))) return c ? set_err(c, VGB_E_ARG, "null argument") : VGB_E_ARG;
+	if (comp_bytes > c->max_chunk_bytes) return set_err(c, VGB_E_ARG, "compressed BAM piece of %llu bytes exceeds max_chunk_bytes", (unsigned long long)comp_bytes);
+	return submit_bam(c, (const uint8_t *)comp, comp_bytes, members, n_members, first, last);
+}
+
 int vgb_sync(vgb_ctx *c)
 {
 	if (!c) return VGB_E_ARG;
@@ -369,6 +390,8 @@ int vgb_sync(vgb_ctx *c)
 	c->sticky_format |= bits;
 	if (c->sticky_format & 8) return set_err(c, VGB_E_FORMAT, "BGZF input: a gzip member is corrupt or does not inflate to the size its trailer states");
 	if (c->sticky_format & 16) return set_err(c, VGB_E_FORMAT, "gzip input: %s", c->gz.err.c_str());
+	if (c->sticky_format & 32)
+		return set_err(c, VGB_E_FORMAT, "BAM input: %s (%llu records with more than 1022 bases)", c->bam.err.c_str(), (unsigned long long)c->bam.long_records);
 	if (c->sticky_format || st.bad_records)
 		return set_err(c, VGB_E_FORMAT, "FASTQ input violates the contract:%s%s%s (%llu bad records)",
 		               (c->sticky_format & 1) ? " truncated record (line count not a multiple of 4);" : "",

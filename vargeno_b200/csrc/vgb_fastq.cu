@@ -167,7 +167,8 @@ int fastq_index_lines(vgb_ctx *c, Chunk &ck, uint64_t nbytes, cudaStream_t st, i
 	return VGB_OK;
 }
 
-// ---- BGZF: the gzip members of a chunk inflated on the device, one warp per member (vgb_inflate.cuh) ----
+// ---- BGZF: the gzip members of a chunk inflated on the device, one warp per member (vgb_inflate.cuh), into `out` (the chunk's
+// text, or the BAM bytes of vgb_submit_bam); a corrupt member sets an error bit in the chunk's meta ----
 // 7 warps of 10.6 KiB (ring + tables) per CTA, three CTAs per SM: 21 members in flight per SM.  Members are claimed one at a time
 // through a counter: their cost varies with what they hold.
 #ifndef VGB_INF_WARPS
@@ -193,7 +194,7 @@ __global__ void __launch_bounds__(INF_WARPS * 32) k_inflate_bgzf(const uint8_t *
 	}
 }
 
-int bgzf_inflate(vgb_ctx *c, Chunk &ck, const uint8_t *d_comp, const BgzfBlock *d_blk, uint32_t n_blk, cudaStream_t st)
+int bgzf_inflate(vgb_ctx *c, Chunk &ck, const uint8_t *d_comp, const BgzfBlock *d_blk, uint32_t n_blk, cudaStream_t st, uint8_t *out)
 {
 	const size_t smem = sizeof(InflateWarp) * INF_WARPS;
 	if (!c->inflate_ready) {
@@ -205,7 +206,7 @@ int bgzf_inflate(vgb_ctx *c, Chunk &ck, const uint8_t *d_comp, const BgzfBlock *
 	}
 	VGB_CUDA(c, cudaMemsetAsync(ck.d_meta + 12, 0, sizeof(uint32_t), st));                // member counter
 	const unsigned grid = (unsigned)std::min<uint64_t>(c->inflate_grid, (n_blk + INF_WARPS - 1) / INF_WARPS);
-	k_inflate_bgzf<<<grid ? grid : 1, INF_WARPS * 32, smem, st>>>(d_comp, d_blk, n_blk, reinterpret_cast<uint8_t *>(ck.d_text), ck.d_meta, ck.d_meta + 12);
+	k_inflate_bgzf<<<grid ? grid : 1, INF_WARPS * 32, smem, st>>>(d_comp, d_blk, n_blk, out, ck.d_meta, ck.d_meta + 12);
 	c->launches++;
 	VGB_CUDA(c, cudaGetLastError());
 	return VGB_OK;

@@ -40,6 +40,24 @@ struct GzStream {
 	std::string err;
 };
 
+struct BamTile;
+struct BamSum;
+// BAM file fed by vgb_submit_bam (vgb_bam.cu): the bytes not consumed yet stay in front of the next call's members, on the device
+struct BamStream {
+	uint8_t *d_buf[2] = {};           // BAM bytes of a call: the unconsumed bytes of the previous call, then its members inflated (d_buf[cur])
+	BamTile *d_tile = nullptr;
+	uint32_t *d_cnt = nullptr, *d_txt = nullptr, *d_scan = nullptr;   // per tile: FASTQ records and text bytes, then their exclusive scans
+	uint32_t *d_rec_off = nullptr, *d_rec_txt = nullptr;              // per FASTQ record: offset in the BAM bytes, offset of its text
+	BamSum *d_sum = nullptr, *h_sum = nullptr;
+	uint64_t cap = 0, carry = 0;      // bytes of each buffer; unconsumed bytes at the front of d_buf[cur]
+	uint64_t tiles = 0, repairs = 0, long_records = 0;
+	uint32_t max_tiles = 0;
+	int32_t n_ref = 0;
+	int cur = 0;
+	bool active = false, header_done = false, failed = false;
+	std::string err;
+};
+
 struct BgzfBlock { uint32_t comp_off, comp_len, out_off, out_len; };   // one gzip member of a chunk: DEFLATE payload in the compressed buffer -> place in the text
 
 struct Chunk {          // one in-flight FASTQ chunk (two slots: copy of chunk i+1 overlaps the kernels of chunk i)
@@ -101,6 +119,7 @@ struct vgb_ctx {
 	bool inflate_ready = false;       // k_inflate_bgzf: shared-memory attribute set, grid sized
 	uint32_t inflate_grid = 0;
 	vgb::GzStream gz;                 // vgb_submit_gzip
+	vgb::BamStream bam;               // vgb_submit_bam
 
 	// host-side statistics
 	uint64_t chunks = 0, chunk_bytes = 0, launches = 0;
@@ -156,13 +175,17 @@ int dev_alloc(vgb_ctx *c, T **p, uint64_t count, bool own = true)
 int index_upload(vgb_ctx *c, const vgb_index_view *v);
 // vgb_fastq.cu
 int fastq_index_lines(vgb_ctx *c, Chunk &ck, uint64_t nbytes, cudaStream_t st, int window = 0, uint64_t ov = 0, int last = 0);
-int bgzf_inflate(vgb_ctx *c, Chunk &ck, const uint8_t *d_comp, const BgzfBlock *d_blk, uint32_t n_blk, cudaStream_t st);
+int bgzf_inflate(vgb_ctx *c, Chunk &ck, const uint8_t *d_comp, const BgzfBlock *d_blk, uint32_t n_blk, cudaStream_t st, uint8_t *out);
 // vgb_gzip.cu
 int submit_gzip(vgb_ctx *c, const uint8_t *comp, uint64_t comp_bytes, int first, int last);
 void gzip_free(vgb_ctx *c);
+// vgb_bam.cu
+int submit_bam(vgb_ctx *c, const uint8_t *comp, uint64_t comp_bytes, const vgb_bgzf_member *mem, uint32_t n_mem, int first, int last);
+void bam_free(vgb_ctx *c);
 // vgb_api.cu
 int process_text(vgb_ctx *c, Chunk &k, uint64_t nbytes, uint64_t first_read_id, int window, uint64_t ov, int last);
 void collect_times(vgb_ctx *c, int slot);
+int bgzf_stage(vgb_ctx *c, Chunk &k, int slot, const uint8_t *comp, uint64_t comp_bytes, const vgb_bgzf_member *mem, uint32_t n_mem, uint64_t *out);
 // vgb_geno.cu
 int geno_launch(vgb_ctx *c, Chunk &ck, uint64_t nbytes, uint64_t first_read_id);
 int geno_prepare(vgb_ctx *c);

@@ -169,6 +169,37 @@ class Genotyper:
                                             1 if last and i + 1 == len(starts) else 0))
         return len(starts)
 
+    def bam_calls(self, buf, own_out: int) -> List[Tuple[np.ndarray, np.ndarray]]:
+        """(compressed members back to back, their vgb_bgzf_member table) of each vgb_submit_bam call of a BAM file image: runs of
+        whole BGZF members with at most `own_out` inflated and max_chunk_bytes compressed bytes (tools/bgzf.scan finds them)"""
+        from .tools import bgzf
+        a = bytes(buf) if isinstance(buf, np.ndarray) else buf
+        mem = [m for m in bgzf.scan(a) if m[3]]
+        own = max(1, min(int(own_out), self.max_chunk_bytes))
+        calls, i = [], 0
+        while i < len(mem):
+            i0, out, comp = i, 0, 0
+            while i < len(mem) and out + mem[i][3] <= own and comp + mem[i][1] <= self.max_chunk_bytes:
+                out += mem[i][3]
+                comp += mem[i][1]
+                i += 1
+            if i == i0:
+                raise ValueError("a BGZF member does not fit one call")
+            calls.append(bgzf.chunk_arrays(a, mem, i0, i))
+        return calls or [(np.zeros(0, np.uint8), np.zeros((0, 3), "<u4"))]
+
+    def submit_bam_call(self, comp: np.ndarray, members: np.ndarray, first: bool, last: bool) -> None:
+        """One vgb_submit_bam call (see bam_calls)"""
+        self._ck(self.L.vgb_submit_bam(self.h, _lib.ptr(comp), comp.size, _lib.ptr(members), members.shape[0], 1 if first else 0, 1 if last else 0))
+
+    def submit_bam(self, buf, own_out: int, first: bool = True, last: bool = True) -> int:
+        """A BAM file image (bytes or uint8 array) through vgb_submit_bam in calls of whole BGZF members (bam_calls); `first` /
+        `last` mark the file's first and last call.  Returns the number of calls."""
+        calls = self.bam_calls(buf, own_out)
+        for k, (comp, tab) in enumerate(calls):
+            self.submit_bam_call(np.ascontiguousarray(comp), np.ascontiguousarray(tab, dtype="<u4"), first and k == 0, last and k + 1 == len(calls))
+        return len(calls)
+
     def submit_device(self, dptr: int, nbytes: int, first_read_id: int = 0) -> None:
         self._ck(self.L.vgb_submit_fastq_device(self.h, C.c_void_p(dptr), nbytes, first_read_id))
 

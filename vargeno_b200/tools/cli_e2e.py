@@ -6,7 +6,8 @@ read loop as the program reports it (index load excluded, reported separately), 
 Everything is made on this box: the S1 index (device builder -> the five files), the reads (device generator -> a file in
 tmpfs, i.e. the page-cache case a warm run sees), the BGZF copy (multi-process zlib level 1, like `bgzip -@`), and a
 single-stream `gzip -1` copy of the first 2 GB, run inflated on the device (vgb_submit_gzip, first GPU only) and, for comparison,
-through host zlib (VGB_HOST_INFLATE=1).  Prints one JSON object per run."""
+through host zlib (VGB_HOST_INFLATE=1), and an unaligned BAM copy of the first 2 GB (the same reads, zlib level 1, one file: one
+GPU; --skip-bam leaves it out).  Prints one JSON object per run."""
 from __future__ import annotations
 
 import argparse
@@ -27,6 +28,7 @@ def main():
     ap.add_argument("--dir", default="/dev/shm/vgb_e2e")
     ap.add_argument("--chunk-mb", type=int, default=512)
     ap.add_argument("--skip-gzip", action="store_true")
+    ap.add_argument("--skip-bam", action="store_true")
     args = ap.parse_args()
     sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
     import bench
@@ -74,6 +76,18 @@ def main():
                 left -= len(blk)
             p.stdin.close()
             p.wait()
+    ubam, n_bam = None, 0
+    if not args.skip_bam:
+        from vargeno_b200.tools import bam
+        ubam = fq + ".bam"
+        n_bam = min(size, (2_000_000_000 // rb) * rb)
+        with open(fq, "rb") as f:
+            raw = bam.ubam_fixed(f.read(n_bam))
+        with open(ubam + ".raw", "wb") as f:
+            f.write(raw)
+        del raw
+        bgzf.compress_file(ubam + ".raw", ubam, procs=max(1, (os.cpu_count() or 2) - 1))
+        os.remove(ubam + ".raw")
 
     def run(tag, path, gpus, n_reads, extra_env=None):
         out = os.path.join(args.dir, "out.vcf")
@@ -109,6 +123,8 @@ def main():
                 if n_small == size:
                     chk["gzip_device_vcf_identical_to_plain"] = d is not None and d == a
                 print(json.dumps(chk), flush=True)
+            if ubam:
+                run("unaligned BAM, first 2 GB of reads, inflated and converted on the device", ubam, gpus, 0)
     shutil.rmtree(args.dir, ignore_errors=True)
 
 

@@ -1,10 +1,11 @@
 """Device-side inflate measured alone: S1-like FASTQ text made on the device and compressed by zlib at two levels, either as BGZF
 pushed through vgb_submit_bgzf (k_inflate_bgzf), or (--mode gzip) as one single gzip stream pushed through vgb_submit_gzip in
-pieces (the sub-stream pipeline of csrc/vgb_gzip.cu).  Prints the rate at which text comes out of the inflate + framing kernels
+pieces (the sub-stream pipeline of csrc/vgb_gzip.cu), or (--mode bam) as unaligned BAM of the same reads at zlib level 1 pushed
+through vgb_submit_bam (members inflated, records framed and converted on the device, csrc/vgb_bam.cu).  Prints the rate at which text comes out of the inflate + framing kernels
 (vgb_stats.gpu_ms_parse: CUDA events around both) and the wall-clock rate of the whole submit loop.  --profile adds one
 repetition under torch.profiler and prints the CUDA time of each kernel (the window chain's share of a round is read there).
 
-    python -m vargeno_b200.tools.inflate_bench [--mode bgzf|gzip] [--reads 4000000] [--chunk-mb 256] [--levels 1,6] [--profile]
+    python -m vargeno_b200.tools.inflate_bench [--mode bgzf|gzip|bam] [--reads 4000000] [--chunk-mb 256] [--levels 1,6] [--profile]
 """
 from __future__ import annotations
 
@@ -30,7 +31,7 @@ def main():
     ap.add_argument("--chunk-mb", type=int, default=256, help="inflated bytes per vgb_submit_bgzf call")
     ap.add_argument("--levels", default="1,6")
     ap.add_argument("--repeats", type=int, default=3)
-    ap.add_argument("--mode", choices=("bgzf", "gzip"), default="bgzf")
+    ap.add_argument("--mode", choices=("bgzf", "gzip", "bam"), default="bgzf")
     ap.add_argument("--piece-mb", type=int, default=64, help="--mode gzip: compressed bytes per vgb_submit_gzip call")
     ap.add_argument("--profile", action="store_true")
     args = ap.parse_args()
@@ -50,6 +51,9 @@ def main():
         dw.synth_batch(g, wl, d, args.reads, 0, 0.005, 0.25, bench.LOWQ_CHARS, bench.REC_ID_WIDTH)
         text = g.d2h(d, args.reads * rb).tobytes()
         g.dfree(d)
+        if args.mode == "bam":
+            _bam_mode(g, text, args)
+            return
         if args.mode == "gzip":
             for level in (int(x) for x in args.levels.split(",")):
                 _gzip_mode(g, text, level, args)
@@ -127,6 +131,43 @@ def _gzip_mode(g, text, level, args):
         rec["kernel_ms"] = {k.split("(")[0]: round(v, 3) for k, v in sorted(ker.items(), key=lambda x: -x[1])[:12]}
         rec["window_chain_share_of_gzip_kernels"] = sum(v for k, v in gz.items() if "k_gz_window" in k) / max(1e-9, sum(gz.values()))
     print(json.dumps(rec), flush=True)
+
+
+def _bam_mode(g, text, args):
+    """uBAM of the reads (level 1, bgzip-sized members); wall-clock reads/s of the submit loop (the BAM kernels are not inside
+    gpu_ms_parse), and the share of 64 KiB tiles the chain walks again (tools/bam.repair_share, the same check as the device)"""
+    import torch
+
+    from vargeno_b200.tools import bam, bgzf
+    t0 = time.time()
+    raw = bam.ubam_fixed(text)
+    span = 65280 * 256
+    with mp.Pool(max(1, (os.cpu_count() or 2) - 1)) as pool:
+        buf = b"".join(pool.imap(_members, [(raw[a:a + span], 1, 65280) for a in range(0, len(raw), span)])) + bgzf.EOF_MEMBER
+    t_comp = time.time() - t0
+    calls = []
+    for comp, tab in g.bam_calls(buf, args.chunk_mb << 20):
+        pin = torch.empty(comp.size, dtype=torch.uint8, pin_memory=True).numpy()
+        pin[:] = comp
+        calls.append((pin, np.ascontiguousarray(tab, dtype="<u4")))
+    n_reads = text.count(b"\n") // 4
+    best = None
+    for rep in range(args.repeats + 1):
+        g.reset()
+        t0 = time.perf_counter()
+        for k, (pin, tab) in enumerate(calls):
+            g.submit_bam_call(pin, tab, k == 0, k + 1 == len(calls))
+        g.sync()
+        dt = time.perf_counter() - t0
+        s1 = g.stats()
+        assert s1["reads"] == n_reads, (s1["reads"], n_reads)
+        if rep and (best is None or dt < best[0]):
+            best = (dt, s1["gpu_ms_parse"], s1["gpu_ms_geno"])
+    tiles, repaired = bam.repair_share(raw[:64 << 20])
+    print(json.dumps({"mode": "bam", "zlib_level": 1, "text_bytes": len(text), "bam_bytes": len(raw), "bgzf_bytes": len(buf), "calls": len(calls),
+                      "compress_s": round(t_comp, 1), "wall_s": best[0], "wall_reads_per_s": n_reads / best[0], "wall_text_gb_per_s": len(text) / best[0] / 1e9,
+                      "framing_ms": best[1], "geno_ms": best[2], "tiles_first_64MiB": tiles, "tiles_repaired": repaired,
+                      "repair_share": repaired / max(1, tiles)}), flush=True)
 
 
 if __name__ == "__main__":
