@@ -180,7 +180,13 @@ int  vgb_submit_gzip(vgb_ctx *ctx, const void *comp, uint64_t comp_bytes, int fi
  * of the members is not verified. */
 int  vgb_submit_bam(vgb_ctx *ctx, const void *comp, uint64_t comp_bytes, const vgb_bgzf_member *members, uint32_t n_members, int first, int last);
 int  vgb_sync(vgb_ctx *ctx);
-int  vgb_reset_counts(vgb_ctx *ctx);              /* zero the pileup counters, statistics and the trace */
+int  vgb_reset_counts(vgb_ctx *ctx);              /* zero the pileup counters, statistics and the trace; an unfinished gzip or BAM input goes on */
+/* End the current sample: waits for all work of the context, does what vgb_reset_counts does, and drops an unfinished gzip stream
+ * (bit cursor, unconsumed bytes, decode window, the text carried for records that span streams, its error) and an unfinished BAM
+ * file (carried bytes, header, its error) without running or reporting them.  The index, the pinned buffers and the device
+ * allocations stay.  The next submit starts a new input: a vgb_submit_gzip or vgb_submit_bam call without `first` is then
+ * VGB_E_ARG.  For a cohort, one index upload serves every sample: submit, vgb_sync, vgb_call, vgb_reset_sample. */
+int  vgb_reset_sample(vgb_ctx *ctx);
 int  vgb_fetch_read_results(vgb_ctx *ctx, vgb_read_result *out, uint64_t cap, uint64_t *n);   /* needs VGB_CFG_TRACE */
 
 /* ---- probes: query_ref_dict / query_snp_dict / check_block_size / BloomFilter::check_value for a batch of

@@ -52,7 +52,7 @@ SYMBOLS = ["vgb_abi_version", "vgb_ctx_create", "vgb_ctx_destroy", "vgb_last_err
            "vgb_synth_reads_device", "vgb_device_alloc", "vgb_device_free", "vgb_memcpy_d2h", "vgb_memcpy_h2d",
            "vgb_build_index_device", "vgb_free_index_device", "vgb_index_upload_device", "vgb_synth_genome_device",
            "vgb_memcpy_d2d", "vgb_memset_device", "vgb_comm_init", "vgb_build_ref_lite_bf_device", "vgb_build_snp_bf_ucsc_device", "vgb_submit_bgzf",
-           "vgb_submit_gzip", "vgb_submit_bam"]
+           "vgb_submit_gzip", "vgb_submit_bam", "vgb_reset_sample"]
 
 _lib = None
 
@@ -80,6 +80,7 @@ def load():
         "vgb_submit_fastq_device": (i32, [vp, vp, u64, u64]),
         "vgb_sync": (i32, [vp]),
         "vgb_reset_counts": (i32, [vp]),
+        "vgb_reset_sample": (i32, [vp]),
         "vgb_fetch_read_results": (i32, [vp, vp, u64, C.POINTER(u64)]),
         "vgb_lookup_kmers": (i32, [vp, vp, u64, vp]),
         "vgb_allreduce_pileup": (i32, [vp]),

@@ -12,6 +12,7 @@
 
 #include <algorithm>
 #include <atomic>
+#include <cerrno>
 #include <chrono>
 #include <cmath>
 #include <cstdio>
@@ -19,6 +20,7 @@
 #include <cstring>
 #include <fstream>
 #include <mutex>
+#include <set>
 #include <thread>
 
 namespace vgh {
@@ -982,24 +984,13 @@ int rewrite_vcf(const std::string &vcf_in, const std::string &vcf_out, const std
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// the command
+// the commands
 // ---------------------------------------------------------------------------------------------------------------
-int run_geno(const std::string &prefix, const std::string &fastq, const std::string &vcf_in, const std::string &vcf_out,
-             int n_gpus, uint64_t chunk_bytes, bool verbose)
+// One context per GPU 0 .. n_gpus - 1 (world_size 1), created and loaded concurrently.  On failure the error is printed, every
+// context is destroyed and ctxs is left empty.
+static bool open_contexts(const IndexFiles &ix, int n_gpus, uint64_t chunk_bytes, std::vector<vgb_ctx *> &ctxs)
 {
-	using clk = std::chrono::steady_clock;
-	const auto t0 = clk::now();
-	auto secs = [&](clk::time_point a) { return std::chrono::duration<double>(clk::now() - a).count(); };
-	std::string err;
-	IndexFiles ix;
-	if (!ix.open(prefix, err)) { fprintf(stderr, "vargeno-b200: %s\n", err.c_str()); return EXIT_FAILURE; }
-	fprintf(stderr, "Initializing...\n");
-
-	// one context per GPU, created and loaded concurrently.  The collective NCCL initialisation starts only after every
-	// rank has its context and its index (vgb_comm_init): a rank that fails early cannot leave the others blocked
-	unsigned char uid[128];
-	if (n_gpus > 1 && vgb_nccl_unique_id(uid) != VGB_OK) { fprintf(stderr, "vargeno-b200: %s\n", vgb_last_error(nullptr)); return EXIT_FAILURE; }
-	std::vector<vgb_ctx *> ctxs(n_gpus, nullptr);
+	ctxs.assign(n_gpus, nullptr);
 	std::vector<int> rcs(n_gpus, 0);
 	std::vector<std::string> errs(n_gpus);
 	{
@@ -1029,8 +1020,31 @@ int run_geno(const std::string &prefix, const std::string &fastq, const std::str
 		if (rcs[r]) {
 			fprintf(stderr, "vargeno-b200: GPU %d: %s\n", r, errs[r].c_str());
 			for (auto c : ctxs) vgb_ctx_destroy(c);
-			return EXIT_FAILURE;
+			ctxs.clear();
+			return false;
 		}
+	return true;
+}
+
+int run_geno(const std::string &prefix, const std::string &fastq, const std::string &vcf_in, const std::string &vcf_out,
+             int n_gpus, uint64_t chunk_bytes, bool verbose)
+{
+	using clk = std::chrono::steady_clock;
+	const auto t0 = clk::now();
+	auto secs = [&](clk::time_point a) { return std::chrono::duration<double>(clk::now() - a).count(); };
+	std::string err;
+	IndexFiles ix;
+	if (!ix.open(prefix, err)) { fprintf(stderr, "vargeno-b200: %s\n", err.c_str()); return EXIT_FAILURE; }
+	fprintf(stderr, "Initializing...\n");
+
+	// The collective NCCL initialisation starts only after every rank has its context and its index (vgb_comm_init): a rank
+	// that fails early cannot leave the others blocked
+	unsigned char uid[128];
+	if (n_gpus > 1 && vgb_nccl_unique_id(uid) != VGB_OK) { fprintf(stderr, "vargeno-b200: %s\n", vgb_last_error(nullptr)); return EXIT_FAILURE; }
+	std::vector<vgb_ctx *> ctxs;
+	if (!open_contexts(ix, n_gpus, chunk_bytes, ctxs)) return EXIT_FAILURE;
+	std::vector<int> rcs(n_gpus, 0);
+	std::vector<std::string> errs(n_gpus);
 	if (n_gpus > 1) {
 		std::vector<std::thread> th;
 		for (int r = 0; r < n_gpus; r++)
@@ -1075,6 +1089,156 @@ int run_geno(const std::string &prefix, const std::string &fastq, const std::str
 	if (rc != VGB_OK) { fprintf(stderr, "vargeno-b200: %s\n", err.c_str()); return EXIT_FAILURE; }
 	printf("Time: %f sec\n", secs(t0));
 	return EXIT_SUCCESS;
+}
+
+// `geno-samples`: a cohort.  The index is loaded once per GPU, each GPU takes whole samples (largest first), and every sample
+// gets the VCF `geno` writes for it alone.
+namespace {
+struct Sample { std::string name, reads; uint64_t bytes = 0; };
+
+bool name_char(char ch)
+{
+	return (ch >= 'A' && ch <= 'Z') || (ch >= 'a' && ch <= 'z') || (ch >= '0' && ch <= '9') || ch == '.' || ch == '_' || ch == '-';
+}
+
+// one sample per line, `name<TAB>reads`; blank lines and lines starting with '#' are skipped.  The first problem fails the sheet
+// with its line number.  Touches no device and no index file.
+bool read_sample_sheet(const std::string &path, std::vector<Sample> &out, std::string &err)
+{
+	std::ifstream in(path);
+	if (!in.good()) { err = "cannot open " + path; return false; }
+	std::set<std::string> seen;
+	std::string line;
+	for (int ln = 1; std::getline(in, line); ln++) {
+		if (!line.empty() && line.back() == '\r') line.pop_back();
+		if (line.empty() || line[0] == '#') continue;
+		auto bad = [&](const std::string &what) { err = path + ":" + std::to_string(ln) + ": " + what; return false; };
+		const size_t tab = line.find('\t');
+		if (tab == std::string::npos) return bad("expected <name><TAB><reads>");
+		Sample s;
+		s.name = line.substr(0, tab);
+		s.reads = line.substr(tab + 1);
+		if (s.name.empty()) return bad("empty sample name");
+		if (!std::all_of(s.name.begin(), s.name.end(), name_char)) return bad("sample name '" + s.name + "' is not made of [A-Za-z0-9._-]");
+		if (!seen.insert(s.name).second) return bad("sample name '" + s.name + "' appears twice");
+		if (s.reads.find('\t') != std::string::npos) return bad("more than two columns");
+		size_t n = 0;
+		for (const std::string &p : split(s.reads, ',')) {       // the list as stream_fastq reads it
+			if (p.empty()) continue;
+			struct stat st;
+			if (stat(p.c_str(), &st) != 0) return bad("reads file " + p + " does not exist");
+			if (S_ISREG(st.st_mode)) s.bytes += (uint64_t)st.st_size;
+			n++;
+		}
+		if (n == 0) return bad("no reads file");
+		out.push_back(s);
+	}
+	if (out.empty()) { err = path + ": no samples"; return false; }
+	return true;
+}
+
+// the directory and any missing parent (mkdir -p); false if it cannot be made or a file of that name is in the way
+bool make_dirs(const std::string &path)
+{
+	for (size_t i = 1; i <= path.size(); i++) {
+		if (i < path.size() && path[i] != '/') continue;
+		if (mkdir(path.substr(0, i).c_str(), 0777) != 0 && errno != EEXIST) return false;
+	}
+	struct stat st;
+	return stat(path.c_str(), &st) == 0 && S_ISDIR(st.st_mode);
+}
+}  // namespace
+
+int run_geno_samples(const std::string &prefix, const std::string &sheet, const std::string &vcf_in, const std::string &out_dir,
+                     int n_gpus, uint64_t chunk_bytes, bool verbose)
+{
+	using clk = std::chrono::steady_clock;
+	const auto t0 = clk::now();
+	auto secs = [](clk::time_point a) { return std::chrono::duration<double>(clk::now() - a).count(); };
+	std::string err;
+	std::vector<Sample> samples;
+	if (!read_sample_sheet(sheet, samples, err)) { fprintf(stderr, "vargeno-b200: %s\n", err.c_str()); return EXIT_FAILURE; }
+	if (!make_dirs(out_dir)) { fprintf(stderr, "vargeno-b200: cannot create the directory %s\n", out_dir.c_str()); return EXIT_FAILURE; }
+	std::stable_sort(samples.begin(), samples.end(), [](const Sample &a, const Sample &b) { return a.bytes > b.bytes; });
+	IndexFiles ix;
+	if (!ix.open(prefix, err)) { fprintf(stderr, "vargeno-b200: %s\n", err.c_str()); return EXIT_FAILURE; }
+	fprintf(stderr, "Initializing...\n");
+	// a sample never spans GPUs: no communicator, and a cohort smaller than --gpus leaves GPUs idle
+	const int n_ctx = std::min<int>(n_gpus, (int)samples.size());
+	std::vector<vgb_ctx *> ctxs;
+	if (!open_contexts(ix, n_ctx, chunk_bytes, ctxs)) return EXIT_FAILURE;
+	const double t_load = secs(t0);
+	fprintf(stderr, "Processing...\n");
+
+	std::atomic<size_t> next(0);
+	std::atomic<int> failed(0), fatal(0);
+	std::vector<std::string> fatal_err(n_ctx);
+	auto report = [&](const Sample &s, int g, bool ok, const vgb_stats &st, double reads_s, double write_s, const std::string &e) {
+		if (!ok) {
+			unlink((out_dir + "/" + s.name + ".vcf").c_str());   // a VCF of an earlier run must not pass for this one
+			fprintf(stderr, "vargeno-b200: sample %s: %s\n", s.name.c_str(), e.c_str());
+			failed++;
+		}
+		if (verbose)
+			fprintf(stderr, "{\"name\": \"%s\", \"gpu\": %d, \"reads\": %llu, \"placed\": %llu, \"reads_s\": %.3f, \"write_s\": %.3f, \"ok\": %s}\n",
+			        s.name.c_str(), g, (unsigned long long)st.reads, (unsigned long long)st.placed, reads_s, write_s, ok ? "true" : "false");
+	};
+	auto worker = [&](int g) {
+		vgb_ctx *ctx = ctxs[g];
+		const std::vector<vgb_ctx *> one{ ctx };
+		uint64_t n = 0;
+		std::vector<uint32_t> pos;                              // site positions depend on the index only
+		if (vgb_site_count(ctx, &n) == VGB_OK) pos.resize(n);
+		if (pos.size() != n || vgb_fetch_sites(ctx, pos.data(), nullptr, nullptr, nullptr, n) != VGB_OK) { fatal_err[g] = vgb_last_error(ctx); fatal = 1; return; }
+		std::thread writer;                                     // the VCF rewrite of the previous sample runs under this one's reads
+		for (;;) {
+			const size_t i = next.fetch_add(1);
+			if (i >= samples.size() || fatal.load()) break;
+			const Sample &s = samples[i];
+			const auto t1 = clk::now();
+			std::vector<uint8_t> gt(n);
+			std::vector<double> conf(n);
+			vgb_stats st{};
+			uint64_t n_chunks = 0;
+			std::string e;
+			int rc = stream_fastq(one, s.reads, chunk_bytes, n_chunks, e);
+			if (rc == VGB_OK && (rc = vgb_sync(ctx)) != VGB_OK) e = vgb_last_error(ctx);
+			if (rc == VGB_OK && (rc = vgb_get_stats(ctx, &st)) != VGB_OK) e = vgb_last_error(ctx);
+			if (rc == VGB_OK && (rc = vgb_call(ctx, gt.data(), conf.data(), n)) != VGB_OK) e = vgb_last_error(ctx);
+			const double reads_s = secs(t1);
+			if (rc == VGB_E_CUDA || rc == VGB_E_INDEX) { fatal_err[g] = e; fatal = 1; break; }
+			if (vgb_reset_sample(ctx) != VGB_OK) { fatal_err[g] = vgb_last_error(ctx); fatal = 1; break; }
+			if (writer.joinable()) writer.join();               // at most one sample per context waits for its VCF
+			if (rc != VGB_OK) { report(s, g, false, st, reads_s, 0, e); continue; }
+			writer = std::thread([&, g, i, st, reads_s, gt = std::move(gt), conf = std::move(conf)]() {
+				const Sample &s = samples[i];
+				const auto t2 = clk::now();
+				const std::string out = out_dir + "/" + s.name + ".vcf", tmp = out + ".tmp";
+				std::unordered_map<std::string, Call> calls;
+				calls_to_map(pos.data(), gt.data(), conf.data(), n, ix.chr, calls);
+				std::string we;
+				int wrc = rewrite_vcf(vcf_in, tmp, calls, we);
+				if (wrc == VGB_OK && rename(tmp.c_str(), out.c_str()) != 0) { wrc = VGB_E_ARG; we = "cannot rename " + tmp + " to " + out; }
+				if (wrc != VGB_OK) unlink(tmp.c_str());
+				report(s, g, wrc == VGB_OK, st, reads_s, secs(t2), we);
+			});
+		}
+		if (writer.joinable()) writer.join();
+	};
+	{
+		std::vector<std::thread> th;
+		for (int g = 0; g < n_ctx; g++) th.emplace_back(worker, g);
+		for (auto &t : th) t.join();
+	}
+	for (auto c : ctxs) vgb_ctx_destroy(c);
+	if (fatal.load()) {
+		for (int g = 0; g < n_ctx; g++) if (!fatal_err[g].empty()) fprintf(stderr, "vargeno-b200: GPU %d: %s\n", g, fatal_err[g].c_str());
+		return EXIT_FAILURE;
+	}
+	if (verbose)
+		fprintf(stderr, "{\"gpus\": %d, \"samples\": %zu, \"failed\": %d, \"load_s\": %.3f, \"total_s\": %.3f}\n", n_ctx, samples.size(), failed.load(), t_load, secs(t0));
+	printf("Time: %f sec\n", secs(t0));
+	return failed.load() ? EXIT_FAILURE : EXIT_SUCCESS;
 }
 
 }  // namespace vgh

@@ -62,6 +62,10 @@ int rewrite_vcf(const std::string &vcf_in, const std::string &vcf_out, const std
 // the whole `geno` command on n_gpus devices of this node; returns process exit status
 int run_geno(const std::string &prefix, const std::string &fastq, const std::string &vcf_in, const std::string &vcf_out,
              int n_gpus, uint64_t chunk_bytes, bool verbose);
+// the whole `geno-samples` command: every sample of the sheet (`name<TAB>reads` per line) to <out_dir>/<name>.vcf, the index
+// loaded once on each of min(n_gpus, samples) devices; returns process exit status (1 if any sample failed)
+int run_geno_samples(const std::string &prefix, const std::string &sheet, const std::string &vcf_in, const std::string &out_dir,
+                     int n_gpus, uint64_t chunk_bytes, bool verbose);
 
 // the whole `index` command: FASTA + VCF text -> device builder -> the five index files (index_host.cpp)
 // dump_parse: write the parsed contigs / SNP lines as text to that file and stop before the device step (host-logic tests)

@@ -21,6 +21,13 @@ static void print_help()
 	fprintf(stderr, "        (BAM, unaligned or aligned: the reads `samtools fastq` gives, inflated and converted on the GPU; each file\n"
 	                "         on one GPU, largest first; a list may not mix BAM and other files; VGB_HOST_INFLATE and\n"
 	                "         VGB_SEQUENTIAL_READER do not apply)\n");
+	fprintf(stderr, "geno-samples  Genotype a cohort (B200)  <index_prefix> <samples.tsv> <input SNPs in VCF> <output dir> "
+	                "[--gpus N] [--chunk-mb M] [--verbose]\n");
+	fprintf(stderr, "        (samples.tsv: one sample per line, <name><TAB><reads>, reads as for geno; names of [A-Za-z0-9._-], unique;\n"
+	                "         '#' lines and blank lines skipped.  Writes <output dir>/<name>.vcf, the file geno writes for that sample.\n"
+	                "         The index is loaded once per GPU and each GPU takes whole samples, largest first: a sample never\n"
+	                "         spans GPUs, so a cohort smaller than --gpus leaves GPUs idle.  A sample whose input fails gets no VCF\n"
+	                "         and the exit status is 1; the other samples go on)\n");
 	fprintf(stderr, "filt    Keep the reference-dictionary entries near SNPs   <ref.dict> <snp_locs> <out.dict>   (the reference's hidden `filt`)\n");
 	fprintf(stderr, "index   Build the index (B200)         <input FASTA> <input SNPs in VCF> <index_prefix> [--gpu D] [--no-lite] [--verbose]\n");
 	fprintf(stderr, "        (the same files as the reference's `vargeno index`, byte for byte; --no-lite skips the 2.3 GB .ref.bf.lite.bf that nothing reads)\n");
@@ -30,7 +37,7 @@ int main(int argc, const char *argv[])
 {
 	if (argc < 2) { print_help(); return 0; }
 	const std::string opt = argv[1];
-	if (opt == "geno") {
+	if (opt == "geno" || opt == "geno-samples") {
 		std::string pos[4];
 		int npos = 0, gpus = 1;
 		uint64_t chunk_mb = 256;
@@ -43,6 +50,7 @@ int main(int argc, const char *argv[])
 			else npos++;
 		}
 		if (npos != 4 || gpus < 1 || chunk_mb < 1 || chunk_mb > 4000) { print_help(); return EXIT_FAILURE; }   // arg_check, src/qv.cc:1875-1881
+		if (opt == "geno-samples") return vgh::run_geno_samples(pos[0], pos[1], pos[2], pos[3], gpus, chunk_mb << 20, verbose);
 		return vgh::run_geno(pos[0], pos[1], pos[2], pos[3], gpus, chunk_mb << 20, verbose);
 	}
 	if (opt == "index") {

@@ -420,6 +420,22 @@ int vgb_reset_counts(vgb_ctx *c)
 	return VGB_OK;
 }
 
+int vgb_reset_sample(vgb_ctx *c)
+{
+	if (!c) return VGB_E_ARG;
+	cudaSetDevice(c->device);
+	VGB_CUDA(c, cudaStreamSynchronize(c->tail_stream));
+	VGB_CUDA(c, cudaStreamSynchronize(c->copy_stream));
+	VGB_CUDA(c, cudaStreamSynchronize(c->stream));
+	collect_times(c, 0);                                     // the last chunks' event times belong to the sample that ends here
+	collect_times(c, 1);
+	const int rc = vgb_reset_counts(c);
+	if (rc != VGB_OK) return rc;
+	gzip_reset(c);
+	bam_reset(c);
+	return VGB_OK;
+}
+
 int vgb_fetch_read_results(vgb_ctx *c, vgb_read_result *out, uint64_t cap, uint64_t *n)
 {
 	if (!c || !n) return VGB_E_ARG;

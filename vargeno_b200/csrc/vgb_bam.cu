@@ -128,6 +128,13 @@ void bam_free(vgb_ctx *c)
 	z = BamStream();
 }
 
+void bam_reset(vgb_ctx *c)
+{
+	BamStream &z = c->bam;
+	z.active = false; z.failed = false; z.err.clear();
+	z.header_done = false; z.carry = 0; z.n_ref = 0; z.cur = 0; z.long_records = 0;
+}
+
 static int bam_readback(vgb_ctx *c)
 {
 	BamStream &z = c->bam;

@@ -187,6 +187,13 @@ void gzip_free(vgb_ctx *c)
 	z = GzStream();
 }
 
+void gzip_reset(vgb_ctx *c)
+{
+	GzStream &z = c->gz;
+	z.active = false; z.failed = false; z.err.clear();
+	z.state = GZ_S_HEADER; z.avail = 0; z.cur = 0; z.members = 0; z.member_text = 0; z.member_crc = 0; z.dec_avail = 0; z.tail_len = 0;
+}
+
 // One round at the cursor: ns sub-streams with `cap` output symbols each; the text goes to the next chunk slot.  *progress: the
 // cursor moved.
 static int gz_round(vgb_ctx *c, uint32_t ns, uint32_t cap, bool *progress)

@@ -179,9 +179,11 @@ int bgzf_inflate(vgb_ctx *c, Chunk &ck, const uint8_t *d_comp, const BgzfBlock *
 // vgb_gzip.cu
 int submit_gzip(vgb_ctx *c, const uint8_t *comp, uint64_t comp_bytes, int first, int last);
 void gzip_free(vgb_ctx *c);
+void gzip_reset(vgb_ctx *c);      // vgb_reset_sample: drop the stream, keep the buffers
 // vgb_bam.cu
 int submit_bam(vgb_ctx *c, const uint8_t *comp, uint64_t comp_bytes, const vgb_bgzf_member *mem, uint32_t n_mem, int first, int last);
 void bam_free(vgb_ctx *c);
+void bam_reset(vgb_ctx *c);       // vgb_reset_sample: drop the file, keep the buffers
 // vgb_api.cu
 int process_text(vgb_ctx *c, Chunk &k, uint64_t nbytes, uint64_t first_read_id, int window, uint64_t ov, int last);
 void collect_times(vgb_ctx *c, int slot);

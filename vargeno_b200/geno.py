@@ -209,6 +209,11 @@ class Genotyper:
     def reset(self) -> None:
         self._ck(self.L.vgb_reset_counts(self.h))
 
+    def reset_sample(self) -> None:
+        """vgb_reset_sample: end the current sample (counters, statistics, trace, and any unfinished gzip or BAM input) and keep
+        the index, so that the next sample is genotyped as if it were the first"""
+        self._ck(self.L.vgb_reset_sample(self.h))
+
     def read_results(self) -> np.ndarray:
         n = C.c_uint64()
         self._ck(self.L.vgb_fetch_read_results(self.h, None, 0, C.byref(n)))
