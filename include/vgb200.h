@@ -189,6 +189,28 @@ int  vgb_reset_counts(vgb_ctx *ctx);              /* zero the pileup counters, s
 int  vgb_reset_sample(vgb_ctx *ctx);
 int  vgb_fetch_read_results(vgb_ctx *ctx, vgb_read_result *out, uint64_t cap, uint64_t *n);   /* needs VGB_CFG_TRACE */
 
+/* ---- output VCF: replaces the rewrite of src/qv.cc:1628-1747 (the host's calls_to_map + rewrite_vcf, which stay as the
+ *      reference of `vargeno-b200 vcf-rewrite`) ----
+ * Output arrives in rounds through a callback: fn(user, bytes, n) gets pinned memory that is valid during the call only; it
+ * returns 0 to go on (anything else ends the call with VGB_E_ARG).  Round k is handed over while the device makes round k + 1. */
+typedef int (*vgb_write_fn)(void *user, const void *bytes, uint64_t n);
+/* The input SNP VCF, parsed once (one scan of the bytes; records whose CHROM + POS matches no site of the uploaded index are left
+ * out) and uploaded beside the index: its bytes plus about 16 B per record.  Contigs as the index's .chrlens lists them.  Needs the
+ * index.  A line longer than 64 MiB is VGB_E_FORMAT.  The caller's bytes may be released when the call returns. */
+int  vgb_vcf_template(vgb_ctx *ctx, const char *vcf, uint64_t nbytes, const char *const *contig_names, const uint64_t *contig_lens, uint32_t n_contigs);
+/* the template of src (another context, same index) copied to dst device to device, without parsing again */
+int  vgb_vcf_template_copy(vgb_ctx *dst, vgb_ctx *src);
+/* One sample's VCF from its calls: gtype per site as vgb_call gives it (0 none 1 ref 2 alt 3 het) and gq per site, the
+ * (int)(-1 * 10 * log(confidence)) the host computes (src/qv.cc:1681; the device never evaluates log).  The bytes are those
+ * rewrite_vcf writes; with bgzf != 0 they come compressed as BGZF members (SAM specification 4.1, at most 65280 bytes of text
+ * each) and the 28-byte end-of-file member.  A VCF error that depends on the sample's calls (the first failing called record,
+ * as rewrite_vcf meets it) is VGB_E_FORMAT with rewrite_vcf's message, before any byte is handed over.  text_bytes (may be NULL):
+ * size of the uncompressed VCF. */
+int  vgb_vcf_write(vgb_ctx *ctx, const uint8_t *gtype, const int32_t *gq, uint64_t n_sites, int bgzf, vgb_write_fn fn, void *user, uint64_t *text_bytes);
+/* BGZF members of any text (host memory, or device memory with text_on_device), 65280 bytes per member, then the end-of-file
+ * member if eof, through fn in rounds as above */
+int  vgb_deflate_bgzf(vgb_ctx *ctx, const void *text, uint64_t nbytes, int text_on_device, int eof, vgb_write_fn fn, void *user);
+
 /* ---- probes: query_ref_dict / query_snp_dict / check_block_size / BloomFilter::check_value for a batch of
  *      packed k-mers (src/qv.cc:206-264,385-411; src/generate_bf.h:112-121) ---- */
 int  vgb_lookup_kmers(vgb_ctx *ctx, const uint64_t *kmers, uint64_t n, vgb_hit *out);

@@ -52,7 +52,11 @@ SYMBOLS = ["vgb_abi_version", "vgb_ctx_create", "vgb_ctx_destroy", "vgb_last_err
            "vgb_synth_reads_device", "vgb_device_alloc", "vgb_device_free", "vgb_memcpy_d2h", "vgb_memcpy_h2d",
            "vgb_build_index_device", "vgb_free_index_device", "vgb_index_upload_device", "vgb_synth_genome_device",
            "vgb_memcpy_d2d", "vgb_memset_device", "vgb_comm_init", "vgb_build_ref_lite_bf_device", "vgb_build_snp_bf_ucsc_device", "vgb_submit_bgzf",
-           "vgb_submit_gzip", "vgb_submit_bam", "vgb_reset_sample"]
+           "vgb_submit_gzip", "vgb_submit_bam", "vgb_reset_sample", "vgb_vcf_template", "vgb_vcf_template_copy", "vgb_vcf_write",
+           "vgb_deflate_bgzf"]
+
+# int (*vgb_write_fn)(void *user, const void *bytes, uint64_t n)
+WRITE_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_uint64)
 
 _lib = None
 
@@ -107,6 +111,10 @@ def load():
         "vgb_submit_gzip": (i32, [vp, vp, u64, i32, i32]),
         "vgb_submit_bam": (i32, [vp, vp, u64, vp, u32, i32, i32]),
         "vgb_build_ref_lite_bf_device": (i32, [vp, vp, vp, vp, u32, C.POINTER(vp), C.POINTER(u64), C.POINTER(u64)]),
+        "vgb_vcf_template": (i32, [vp, vp, u64, C.POINTER(C.c_char_p), vp, u32]),
+        "vgb_vcf_template_copy": (i32, [vp, vp]),
+        "vgb_vcf_write": (i32, [vp, vp, vp, u64, i32, WRITE_FN, vp, C.POINTER(u64)]),
+        "vgb_deflate_bgzf": (i32, [vp, vp, u64, i32, i32, WRITE_FN, vp]),
     }
     for name in SYMBOLS:
         fn = getattr(L, name)           # AttributeError if the library does not export what the header declares

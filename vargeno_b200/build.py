@@ -19,10 +19,10 @@ LIB = os.path.join(HERE, "libvgb200.so")
 HOST_BIN = os.path.join(HERE, "vargeno-b200")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 
-CU = ["vgb_api.cu", "vgb_index.cu", "vgb_fastq.cu", "vgb_geno.cu", "vgb_call.cu", "vgb_bench.cu", "vgb_build.cu", "vgb_gzip.cu", "vgb_bam.cu"]
+CU = ["vgb_api.cu", "vgb_index.cu", "vgb_fastq.cu", "vgb_geno.cu", "vgb_call.cu", "vgb_bench.cu", "vgb_build.cu", "vgb_gzip.cu", "vgb_bam.cu", "vgb_vcf.cu"]
 CPP = ["vgb_tables.cpp", "vgb_nccl.cpp"]
 HOST_CPP = ["host/vargeno_main.cpp", "host/geno_host.cpp", "host/index_host.cpp"]
-HEADERS = ["vgb_common.cuh", "vgb_internal.h", "vgb_geno8.inl", "vgb_inflate.cuh", "vgb_gzip.cuh", "vgb_bam.cuh", os.path.join("..", "..", "include", "vgb200.h"), "host/geno_host.h"]
+HEADERS = ["vgb_common.cuh", "vgb_internal.h", "vgb_geno8.inl", "vgb_inflate.cuh", "vgb_gzip.cuh", "vgb_bam.cuh", "vgb_deflate.cuh", "vgb_vcf.cuh", os.path.join("..", "..", "include", "vgb200.h"), "host/geno_host.h"]
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC,-ffp-contract=off,-Wall", "-ccbin", "g++", "--fmad=false"] + os.environ.get("VGB_NVCC_DEFINES", "").split()   # A/B builds of compile-time variants (tools/sweep_wgs.py, VGB200_LIB)

@@ -853,22 +853,6 @@ int run_fastq_chunks(const std::string &fastq, uint64_t chunk_bytes, bool timing
 // ---------------------------------------------------------------------------------------------------------------
 // calls + VCF
 // ---------------------------------------------------------------------------------------------------------------
-int collect_calls(vgb_ctx *ctx, const ChrLens &chr, std::unordered_map<std::string, Call> &out, std::string &err)
-{
-	uint64_t n = 0;
-	int rc = vgb_site_count(ctx, &n);
-	if (rc) { err = vgb_last_error(ctx); return rc; }
-	std::vector<uint32_t> pos(n);
-	std::vector<uint8_t> gt(n);
-	std::vector<double> conf(n);
-	if ((rc = vgb_fetch_sites(ctx, pos.data(), nullptr, nullptr, nullptr, n)) || (rc = vgb_call(ctx, gt.data(), conf.data(), n))) {
-		err = vgb_last_error(ctx);
-		return rc;
-	}
-	calls_to_map(pos.data(), gt.data(), conf.data(), n, chr, out);
-	return VGB_OK;
-}
-
 void calls_to_map(const uint32_t *pos, const uint8_t *gt, const double *conf, uint64_t n, const ChrLens &chr, std::unordered_map<std::string, Call> &out)
 {
 	for (uint64_t i = 0; i < n; i++) {                          // position order, like the scan of src/qv.cc:1573-1626
@@ -984,6 +968,112 @@ int rewrite_vcf(const std::string &vcf_in, const std::string &vcf_out, const std
 }
 
 // ---------------------------------------------------------------------------------------------------------------
+// the output VCF on the device (vgb_vcf_template / vgb_vcf_write): the same bytes as rewrite_vcf, BGZF for a name ending in .gz
+// ---------------------------------------------------------------------------------------------------------------
+int upload_vcf_template(const std::vector<vgb_ctx *> &ctxs, const std::string &vcf_in, const ChrLens &chr, std::string &err)
+{
+	// a regular file is mapped; anything else (a FIFO, /dev/stdin from a pipe, <(zcat snps.vcf.gz)) has no size to map and is
+	// read to its end, as rewrite_vcf's ifstream did
+	MappedFile f;
+	std::string piped;
+	const char *data = nullptr;
+	uint64_t size = 0;
+	{
+		struct stat st;
+		if (stat(vcf_in.c_str(), &st) != 0) { err = "Error opening: " + vcf_in; return VGB_E_ARG; }
+		if (S_ISREG(st.st_mode)) {
+			std::string e;
+			if (!f.open(vcf_in, e)) { err = "Error opening: " + vcf_in; return VGB_E_ARG; }
+			data = (const char *)f.data;
+			size = f.size;
+		} else {
+			const int fd = ::open(vcf_in.c_str(), O_RDONLY);
+			if (fd < 0) { err = "Error opening: " + vcf_in; return VGB_E_ARG; }
+			std::vector<char> buf(1u << 20);
+			ssize_t r;
+			while ((r = ::read(fd, buf.data(), buf.size())) > 0) piped.append(buf.data(), (size_t)r);
+			::close(fd);
+			if (r < 0) { err = "read error on " + vcf_in; return VGB_E_ARG; }
+			data = piped.data();
+			size = piped.size();
+		}
+	}
+	std::vector<const char *> names;
+	for (const std::string &n : chr.names) names.push_back(n.c_str());
+	int rc = vgb_vcf_template(ctxs[0], data, size, names.data(), chr.lens.data(), (uint32_t)names.size());
+	if (rc != VGB_OK) { err = vgb_last_error(ctxs[0]); return rc; }
+	for (size_t g = 1; g < ctxs.size(); g++)
+		if ((rc = vgb_vcf_template_copy(ctxs[g], ctxs[0])) != VGB_OK) { err = vgb_last_error(ctxs[g]); return rc; }
+	return VGB_OK;
+}
+
+namespace {
+int append_bytes(void *user, const void *bytes, uint64_t n)
+{
+	static_cast<std::string *>(user)->append(static_cast<const char *>(bytes), n);
+	return 0;
+}
+int fwrite_bytes(void *user, const void *bytes, uint64_t n) { return fwrite(bytes, 1, n, static_cast<FILE *>(user)) == n ? 0 : 1; }
+
+// GQ as rewrite_vcf computes it, on the host with the C library's log (src/qv.cc:1681); 0 for sites that are not called
+std::vector<int32_t> site_gq(const uint8_t *gt, const double *conf, uint64_t n)
+{
+	std::vector<int32_t> gq(n, 0);
+	for (uint64_t i = 0; i < n; i++) if (gt[i]) gq[i] = (int)(-1 * 10 * std::log(conf[i]));
+	return gq;
+}
+
+int vcf_to(vgb_ctx *ctx, const uint8_t *gt, const double *conf, uint64_t n, bool bgzf, vgb_write_fn fn, void *user, std::string &err)
+{
+	const std::vector<int32_t> gq = site_gq(gt, conf, n);
+	const int rc = vgb_vcf_write(ctx, gt, gq.data(), n, bgzf ? 1 : 0, fn, user, nullptr);
+	if (rc != VGB_OK) err = vgb_last_error(ctx);
+	return rc;
+}
+
+// called sites counted as calls_to_map counts them: distinct "name$rel" keys (sites of one key count once)
+uint64_t distinct_called_keys(const uint8_t *gt, vgb_ctx *ctx, uint64_t n, const ChrLens &chr)
+{
+	std::vector<uint32_t> pos(n);
+	if (n && vgb_fetch_sites(ctx, pos.data(), nullptr, nullptr, nullptr, n) != VGB_OK) return 0;
+	std::unordered_map<std::string, uint64_t> name_id;
+	std::vector<uint64_t> keys;
+	std::string name;
+	for (uint64_t i = 0; i < n; i++) {
+		if (!gt[i]) continue;
+		uint64_t rel;
+		chr.locate(pos[i], name, rel);
+		const uint64_t id = name_id.emplace(name, name_id.size()).first->second;
+		keys.push_back(id << 40 | rel);
+	}
+	std::sort(keys.begin(), keys.end());
+	return (uint64_t)(std::unique(keys.begin(), keys.end()) - keys.begin());
+}
+
+bool ends_with_gz(const std::string &s) { return s.size() >= 3 && s.compare(s.size() - 3, 3, ".gz") == 0; }
+
+// one sample's VCF straight into the file (geno)
+int write_vcf_file(vgb_ctx *ctx, const uint8_t *gt, const double *conf, uint64_t n, const std::string &path, std::string &err)
+{
+	FILE *f = fopen(path.c_str(), "wb");
+	if (!f) { err = "cannot write " + path; return VGB_E_ARG; }
+	int rc = vcf_to(ctx, gt, conf, n, ends_with_gz(path), fwrite_bytes, f, err);
+	const bool bad_write = rc == VGB_E_ARG && err == "the output callback failed";
+	if (fclose(f) != 0 || bad_write) { err = "writing the output VCF failed (disk full or I/O error)"; rc = VGB_E_ARG; }
+	return rc;
+}
+
+// bytes to a file: false on any error
+bool write_bytes(const std::string &path, const std::string &bytes)
+{
+	FILE *f = fopen(path.c_str(), "wb");
+	if (!f) return false;
+	const bool ok = fwrite(bytes.data(), 1, bytes.size(), f) == bytes.size();
+	return fclose(f) == 0 && ok;
+}
+}  // namespace
+
+// ---------------------------------------------------------------------------------------------------------------
 // the commands
 // ---------------------------------------------------------------------------------------------------------------
 // One context per GPU 0 .. n_gpus - 1 (world_size 1), created and loaded concurrently.  On failure the error is printed, every
@@ -1057,12 +1147,18 @@ int run_geno(const std::string &prefix, const std::string &fastq, const std::str
 				return EXIT_FAILURE;
 			}
 	}
+	int rc = upload_vcf_template({ ctxs[0] }, vcf_in, ix.chr, err);   // the input VCF, parsed once, beside context 0's index (it writes)
+	if (rc != VGB_OK) {
+		for (auto c : ctxs) vgb_ctx_destroy(c);
+		fprintf(stderr, "vargeno-b200: %s\n", err.c_str());
+		return EXIT_FAILURE;
+	}
 	const double t_load = secs(t0);
 	fprintf(stderr, "Processing...\n");
 
 	const auto t1 = clk::now();
 	uint64_t n_chunks = 0;
-	int rc = stream_fastq(ctxs, fastq, chunk_bytes, n_chunks, err);
+	rc = stream_fastq(ctxs, fastq, chunk_bytes, n_chunks, err);
 	for (int r = 0; rc == VGB_OK && r < n_gpus; r++)
 		if ((rc = vgb_sync(ctxs[r])) != VGB_OK) err = vgb_last_error(ctxs[r]);
 	if (rc == VGB_OK && n_gpus > 1) {                            // one exchange step: sum of the per-SNP counters (SURVEY 8(e))
@@ -1072,9 +1168,15 @@ int run_geno(const std::string &prefix, const std::string &fastq, const std::str
 		for (int r = 0; r < n_gpus; r++) if (rcs[r]) { rc = rcs[r]; err = errs[r]; }
 	}
 	const double t_reads = secs(t1);
-	std::unordered_map<std::string, Call> calls;
-	if (rc == VGB_OK) rc = collect_calls(ctxs[0], ix.chr, calls, err);
-	if (rc == VGB_OK) rc = rewrite_vcf(vcf_in, vcf_out, calls, err);
+	uint64_t n_sites = 0, n_called = 0;
+	if (rc == VGB_OK && (rc = vgb_site_count(ctxs[0], &n_sites)) != VGB_OK) err = vgb_last_error(ctxs[0]);
+	std::vector<uint8_t> gt(n_sites);
+	std::vector<double> conf(n_sites);
+	if (rc == VGB_OK && (rc = vgb_call(ctxs[0], gt.data(), conf.data(), n_sites)) != VGB_OK) err = vgb_last_error(ctxs[0]);
+	const auto t2 = clk::now();
+	if (rc == VGB_OK) rc = write_vcf_file(ctxs[0], gt.data(), conf.data(), n_sites, vcf_out, err);
+	const double t_write = secs(t2);
+	if (verbose) n_called = distinct_called_keys(gt.data(), ctxs[0], n_sites, ix.chr);
 	if (rc == VGB_OK && verbose) {
 		uint64_t reads = 0, placed = 0, lookups = 0;
 		for (auto c : ctxs) {
@@ -1082,8 +1184,8 @@ int run_geno(const std::string &prefix, const std::string &fastq, const std::str
 			if (vgb_get_stats(c, &st) == VGB_OK) { reads += st.reads; placed += st.placed; lookups += st.exact_lookups + st.nbr_query_lookups + st.nbr_scan_reads; }
 		}
 		fprintf(stderr, "{\"gpus\": %d, \"reads\": %llu, \"placed\": %llu, \"kmer_lookups\": %llu, \"chunks\": %llu, \"load_s\": %.3f, \"reads_s\": %.3f, "
-		        "\"reads_per_s\": %.0f, \"calls\": %zu}\n", n_gpus, (unsigned long long)reads, (unsigned long long)placed, (unsigned long long)lookups,
-		        (unsigned long long)n_chunks, t_load, t_reads, reads / (t_reads > 0 ? t_reads : 1), calls.size());
+		        "\"reads_per_s\": %.0f, \"calls\": %llu, \"write_s\": %.3f}\n", n_gpus, (unsigned long long)reads, (unsigned long long)placed,
+		        (unsigned long long)lookups, (unsigned long long)n_chunks, t_load, t_reads, reads / (t_reads > 0 ? t_reads : 1), (unsigned long long)n_called, t_write);
 	}
 	for (auto c : ctxs) vgb_ctx_destroy(c);
 	if (rc != VGB_OK) { fprintf(stderr, "vargeno-b200: %s\n", err.c_str()); return EXIT_FAILURE; }
@@ -1150,7 +1252,7 @@ bool make_dirs(const std::string &path)
 }  // namespace
 
 int run_geno_samples(const std::string &prefix, const std::string &sheet, const std::string &vcf_in, const std::string &out_dir,
-                     int n_gpus, uint64_t chunk_bytes, bool verbose)
+                     int n_gpus, uint64_t chunk_bytes, bool verbose, bool bgzf)
 {
 	using clk = std::chrono::steady_clock;
 	const auto t0 = clk::now();
@@ -1167,6 +1269,12 @@ int run_geno_samples(const std::string &prefix, const std::string &sheet, const 
 	const int n_ctx = std::min<int>(n_gpus, (int)samples.size());
 	std::vector<vgb_ctx *> ctxs;
 	if (!open_contexts(ix, n_ctx, chunk_bytes, ctxs)) return EXIT_FAILURE;
+	if (upload_vcf_template(ctxs, vcf_in, ix.chr, err) != VGB_OK) {       // parsed once, copied to the other GPUs
+		for (auto c : ctxs) vgb_ctx_destroy(c);
+		fprintf(stderr, "vargeno-b200: %s\n", err.c_str());
+		return EXIT_FAILURE;
+	}
+	const std::string ext = bgzf ? ".vcf.gz" : ".vcf";
 	const double t_load = secs(t0);
 	fprintf(stderr, "Processing...\n");
 
@@ -1175,7 +1283,7 @@ int run_geno_samples(const std::string &prefix, const std::string &sheet, const 
 	std::vector<std::string> fatal_err(n_ctx);
 	auto report = [&](const Sample &s, int g, bool ok, const vgb_stats &st, double reads_s, double write_s, const std::string &e) {
 		if (!ok) {
-			unlink((out_dir + "/" + s.name + ".vcf").c_str());   // a VCF of an earlier run must not pass for this one
+			unlink((out_dir + "/" + s.name + ext).c_str());      // a VCF of an earlier run must not pass for this one
 			fprintf(stderr, "vargeno-b200: sample %s: %s\n", s.name.c_str(), e.c_str());
 			failed++;
 		}
@@ -1187,10 +1295,8 @@ int run_geno_samples(const std::string &prefix, const std::string &sheet, const 
 		vgb_ctx *ctx = ctxs[g];
 		const std::vector<vgb_ctx *> one{ ctx };
 		uint64_t n = 0;
-		std::vector<uint32_t> pos;                              // site positions depend on the index only
-		if (vgb_site_count(ctx, &n) == VGB_OK) pos.resize(n);
-		if (pos.size() != n || vgb_fetch_sites(ctx, pos.data(), nullptr, nullptr, nullptr, n) != VGB_OK) { fatal_err[g] = vgb_last_error(ctx); fatal = 1; return; }
-		std::thread writer;                                     // the VCF rewrite of the previous sample runs under this one's reads
+		if (vgb_site_count(ctx, &n) != VGB_OK) { fatal_err[g] = vgb_last_error(ctx); fatal = 1; return; }
+		std::thread writer;                                     // the file write of the previous sample runs under this one's reads
 		for (;;) {
 			const size_t i = next.fetch_add(1);
 			if (i >= samples.size() || fatal.load()) break;
@@ -1208,19 +1314,24 @@ int run_geno_samples(const std::string &prefix, const std::string &sheet, const 
 			const double reads_s = secs(t1);
 			if (rc == VGB_E_CUDA || rc == VGB_E_INDEX) { fatal_err[g] = e; fatal = 1; break; }
 			if (vgb_reset_sample(ctx) != VGB_OK) { fatal_err[g] = vgb_last_error(ctx); fatal = 1; break; }
-			if (writer.joinable()) writer.join();               // at most one sample per context waits for its VCF
+			// the VCF bytes on the device, into host memory; a VCF error of this sample's calls fails this sample only
+			const auto t2 = clk::now();
+			std::string bytes;
+			if (rc == VGB_OK) rc = vcf_to(ctx, gt.data(), conf.data(), n, bgzf, append_bytes, &bytes, e);
+			if (rc == VGB_E_CUDA) { fatal_err[g] = e; fatal = 1; break; }
+			const double vcf_s = secs(t2);
+			if (writer.joinable()) writer.join();               // at most one sample per context waits for its file
 			if (rc != VGB_OK) { report(s, g, false, st, reads_s, 0, e); continue; }
-			writer = std::thread([&, g, i, st, reads_s, gt = std::move(gt), conf = std::move(conf)]() {
+			writer = std::thread([&, g, i, st, reads_s, vcf_s, bytes = std::move(bytes)]() {
 				const Sample &s = samples[i];
-				const auto t2 = clk::now();
-				const std::string out = out_dir + "/" + s.name + ".vcf", tmp = out + ".tmp";
-				std::unordered_map<std::string, Call> calls;
-				calls_to_map(pos.data(), gt.data(), conf.data(), n, ix.chr, calls);
+				const auto t3 = clk::now();
+				const std::string out = out_dir + "/" + s.name + ext, tmp = out + ".tmp";
 				std::string we;
-				int wrc = rewrite_vcf(vcf_in, tmp, calls, we);
+				int wrc = VGB_OK;
+				if (!write_bytes(tmp, bytes)) { wrc = VGB_E_ARG; we = "writing " + tmp + " failed (disk full or I/O error)"; }
 				if (wrc == VGB_OK && rename(tmp.c_str(), out.c_str()) != 0) { wrc = VGB_E_ARG; we = "cannot rename " + tmp + " to " + out; }
 				if (wrc != VGB_OK) unlink(tmp.c_str());
-				report(s, g, wrc == VGB_OK, st, reads_s, secs(t2), we);
+				report(s, g, wrc == VGB_OK, st, reads_s, vcf_s + secs(t3), we);
 			});
 		}
 		if (writer.joinable()) writer.join();

@@ -51,21 +51,22 @@ int stream_fastq_to(ChunkSink &sink, const std::string &path, uint64_t chunk_byt
 int run_fastq_chunks(const std::string &fastq, uint64_t chunk_bytes, bool timing = false, int parallel = 0);   // `vargeno-b200 fastq-chunks <files> [--chunk-bytes B] [--time] [--parallel N]`
 
 // stage F on the host side: device calls -> "chr$pos" -> (gt, conf) map (src/qv.cc:1596-1621)
-int collect_calls(vgb_ctx *ctx, const ChrLens &chr, std::unordered_map<std::string, Call> &out, std::string &err);
-
 void calls_to_map(const uint32_t *pos, const uint8_t *gt, const double *conf, uint64_t n, const ChrLens &chr, std::unordered_map<std::string, Call> &out);
 int run_vcf_rewrite(const std::string &prefix, const std::string &calls_tsv, const std::string &vcf_in, const std::string &vcf_out);   // host-logic tests
 
-// stage G: VCF rewrite (src/qv.cc:1628-1747)
+// stage G: VCF rewrite (src/qv.cc:1628-1747) on the host: the reference of the device writer (vgb_vcf_write), run by `vcf-rewrite`
 int rewrite_vcf(const std::string &vcf_in, const std::string &vcf_out, const std::unordered_map<std::string, Call> &calls, std::string &err);
 
 // the whole `geno` command on n_gpus devices of this node; returns process exit status
 int run_geno(const std::string &prefix, const std::string &fastq, const std::string &vcf_in, const std::string &vcf_out,
              int n_gpus, uint64_t chunk_bytes, bool verbose);
-// the whole `geno-samples` command: every sample of the sheet (`name<TAB>reads` per line) to <out_dir>/<name>.vcf, the index
-// loaded once on each of min(n_gpus, samples) devices; returns process exit status (1 if any sample failed)
+// the whole `geno-samples` command: every sample of the sheet (`name<TAB>reads` per line) to <out_dir>/<name>.vcf (.vcf.gz, BGZF,
+// with bgzf), the index and the VCF template loaded once on each of min(n_gpus, samples) devices; returns process exit status (1 if
+// any sample failed)
 int run_geno_samples(const std::string &prefix, const std::string &sheet, const std::string &vcf_in, const std::string &out_dir,
-                     int n_gpus, uint64_t chunk_bytes, bool verbose);
+                     int n_gpus, uint64_t chunk_bytes, bool verbose, bool bgzf = false);
+// the input VCF parsed once and uploaded as the output template to ctxs[0], copied device to device to the others
+int upload_vcf_template(const std::vector<vgb_ctx *> &ctxs, const std::string &vcf_in, const ChrLens &chr, std::string &err);
 
 // the whole `index` command: FASTA + VCF text -> device builder -> the five index files (index_host.cpp)
 // dump_parse: write the parsed contigs / SNP lines as text to that file and stop before the device step (host-logic tests)

@@ -18,13 +18,14 @@ static void print_help()
 	fprintf(stderr, "        (<input FASTQ>: one file or a comma-separated list read back to back; each plain or gzip; or BAM files only)\n");
 	fprintf(stderr, "        (gzip input is inflated on the GPU: BGZF over all GPUs, single-stream gzip on the first GPU only;\n"
 	                "         pipes and lists that mix plain and gzip files are inflated on the host)\n");
+	fprintf(stderr, "        (the VCF is written on the GPU; an output name ending in .gz gets BGZF, as bgzip writes it)\n");
 	fprintf(stderr, "        (BAM, unaligned or aligned: the reads `samtools fastq` gives, inflated and converted on the GPU; each file\n"
 	                "         on one GPU, largest first; a list may not mix BAM and other files; VGB_HOST_INFLATE and\n"
 	                "         VGB_SEQUENTIAL_READER do not apply)\n");
 	fprintf(stderr, "geno-samples  Genotype a cohort (B200)  <index_prefix> <samples.tsv> <input SNPs in VCF> <output dir> "
-	                "[--gpus N] [--chunk-mb M] [--verbose]\n");
+	                "[--gpus N] [--chunk-mb M] [--bgzf] [--verbose]\n");
 	fprintf(stderr, "        (samples.tsv: one sample per line, <name><TAB><reads>, reads as for geno; names of [A-Za-z0-9._-], unique;\n"
-	                "         '#' lines and blank lines skipped.  Writes <output dir>/<name>.vcf, the file geno writes for that sample.\n"
+	                "         '#' lines and blank lines skipped.  Writes <output dir>/<name>.vcf (--bgzf: <name>.vcf.gz), the file geno writes for that sample.\n"
 	                "         The index is loaded once per GPU and each GPU takes whole samples, largest first: a sample never\n"
 	                "         spans GPUs, so a cohort smaller than --gpus leaves GPUs idle.  A sample whose input fails gets no VCF\n"
 	                "         and the exit status is 1; the other samples go on)\n");
@@ -41,16 +42,17 @@ int main(int argc, const char *argv[])
 		std::string pos[4];
 		int npos = 0, gpus = 1;
 		uint64_t chunk_mb = 256;
-		bool verbose = false;
+		bool verbose = false, bgzf = false;
 		for (int i = 2; i < argc; i++) {
 			if (!strcmp(argv[i], "--gpus") && i + 1 < argc) gpus = atoi(argv[++i]);
 			else if (!strcmp(argv[i], "--chunk-mb") && i + 1 < argc) chunk_mb = strtoull(argv[++i], nullptr, 10);
 			else if (!strcmp(argv[i], "--verbose")) verbose = true;
+			else if (!strcmp(argv[i], "--bgzf") && opt == "geno-samples") bgzf = true;
 			else if (npos < 4) pos[npos++] = argv[i];
 			else npos++;
 		}
 		if (npos != 4 || gpus < 1 || chunk_mb < 1 || chunk_mb > 4000) { print_help(); return EXIT_FAILURE; }   // arg_check, src/qv.cc:1875-1881
-		if (opt == "geno-samples") return vgh::run_geno_samples(pos[0], pos[1], pos[2], pos[3], gpus, chunk_mb << 20, verbose);
+		if (opt == "geno-samples") return vgh::run_geno_samples(pos[0], pos[1], pos[2], pos[3], gpus, chunk_mb << 20, verbose, bgzf);
 		return vgh::run_geno(pos[0], pos[1], pos[2], pos[3], gpus, chunk_mb << 20, verbose);
 	}
 	if (opt == "index") {

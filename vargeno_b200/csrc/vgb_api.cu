@@ -140,6 +140,7 @@ void vgb_ctx_destroy(vgb_ctx *c)
 	}
 	gzip_free(c);
 	bam_free(c);
+	vcf_free(c);
 	cudaFree(c->d_stats); cudaFree(c->d_tables); cudaFree(c->d_trace);
 	for (int i = 0; i < 4; i++) if (c->ev[i]) cudaEventDestroy(c->ev[i]);
 	if (c->stream) cudaStreamDestroy(c->stream);
@@ -434,6 +435,34 @@ int vgb_reset_sample(vgb_ctx *c)
 	gzip_reset(c);
 	bam_reset(c);
 	return VGB_OK;
+}
+
+int vgb_vcf_template(vgb_ctx *c, const char *vcf, uint64_t nbytes, const char *const *contig_names, const uint64_t *contig_lens, uint32_t n_contigs)
+{
+	if (!c || (n_contigs && (!contig_names || !contig_lens))) return VGB_E_ARG;
+	cudaSetDevice(c->device);
+	return vcf_template(c, vcf, nbytes, contig_names, contig_lens, n_contigs);
+}
+
+int vgb_vcf_template_copy(vgb_ctx *dst, vgb_ctx *src)
+{
+	if (!dst || !src) return VGB_E_ARG;
+	cudaSetDevice(dst->device);
+	return vcf_template_copy(dst, src);
+}
+
+int vgb_vcf_write(vgb_ctx *c, const uint8_t *gtype, const int32_t *gq, uint64_t n_sites, int bgzf, vgb_write_fn fn, void *user, uint64_t *text_bytes)
+{
+	if (!c) return VGB_E_ARG;
+	cudaSetDevice(c->device);
+	return vcf_write(c, gtype, gq, n_sites, bgzf, fn, user, text_bytes);
+}
+
+int vgb_deflate_bgzf(vgb_ctx *c, const void *text, uint64_t nbytes, int text_on_device, int eof, vgb_write_fn fn, void *user)
+{
+	if (!c) return VGB_E_ARG;
+	cudaSetDevice(c->device);
+	return deflate_bgzf(c, text, nbytes, text_on_device, eof, fn, user);
 }
 
 int vgb_fetch_read_results(vgb_ctx *c, vgb_read_result *out, uint64_t cap, uint64_t *n)

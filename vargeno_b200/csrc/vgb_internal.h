@@ -58,6 +58,26 @@ struct BamStream {
 	std::string err;
 };
 
+struct VcfRec;
+// output VCF (vgb_vcf.cu): the template of the input VCF, the per-sample arrays and the round buffers
+struct VcfState {
+	uint8_t *d_text = nullptr;        // the VCF bytes, then the header lines as written
+	VcfRec *d_rec = nullptr;
+	uint32_t *d_lists = nullptr;
+	uint64_t text_n = 0, n_rec = 0, n_lists = 0, n_sites = 0;
+	bool ready = false;
+	uint8_t *d_gt = nullptr;          // per site: gtype, GQ
+	int32_t *d_gq = nullptr;
+	uint64_t site_cap = 0;
+	uint32_t *d_len = nullptr;        // per record: output bytes
+	uint64_t *d_off = nullptr, *d_scan = nullptr;   // their exclusive scan; per tile of records: its sum, then its base
+	uint8_t *d_round = nullptr, *d_slots = nullptr, *d_packed = nullptr;   // a round's text, its members (64 KiB slots), packed
+	uint32_t *d_sym = nullptr, *d_msize = nullptr;                        // LZ77 symbols per block; member sizes, offsets
+	unsigned long long *d_misc = nullptr, *h_misc = nullptr;
+	uint8_t *h_out[2] = {};           // pinned: rounds k and k + 1
+	cudaEvent_t ev[2] = {};
+};
+
 struct BgzfBlock { uint32_t comp_off, comp_len, out_off, out_len; };   // one gzip member of a chunk: DEFLATE payload in the compressed buffer -> place in the text
 
 struct Chunk {          // one in-flight FASTQ chunk (two slots: copy of chunk i+1 overlaps the kernels of chunk i)
@@ -120,6 +140,7 @@ struct vgb_ctx {
 	uint32_t inflate_grid = 0;
 	vgb::GzStream gz;                 // vgb_submit_gzip
 	vgb::BamStream bam;               // vgb_submit_bam
+	vgb::VcfState vcf;                // vgb_vcf_template / vgb_vcf_write / vgb_deflate_bgzf
 
 	// host-side statistics
 	uint64_t chunks = 0, chunk_bytes = 0, launches = 0;
@@ -184,6 +205,12 @@ void gzip_reset(vgb_ctx *c);      // vgb_reset_sample: drop the stream, keep the
 int submit_bam(vgb_ctx *c, const uint8_t *comp, uint64_t comp_bytes, const vgb_bgzf_member *mem, uint32_t n_mem, int first, int last);
 void bam_free(vgb_ctx *c);
 void bam_reset(vgb_ctx *c);       // vgb_reset_sample: drop the file, keep the buffers
+// vgb_vcf.cu
+int vcf_template(vgb_ctx *c, const char *vcf, uint64_t n, const char *const *names, const uint64_t *lens, uint32_t n_contigs);
+int vcf_template_copy(vgb_ctx *dst, vgb_ctx *src);
+int vcf_write(vgb_ctx *c, const uint8_t *gt, const int32_t *gq, uint64_t n_sites, int bgzf, vgb_write_fn fn, void *user, uint64_t *text_bytes);
+int deflate_bgzf(vgb_ctx *c, const void *text, uint64_t nbytes, int on_device, int eof, vgb_write_fn fn, void *user);
+void vcf_free(vgb_ctx *c);
 // vgb_api.cu
 int process_text(vgb_ctx *c, Chunk &k, uint64_t nbytes, uint64_t first_read_id, int window, uint64_t ov, int last);
 void collect_times(vgb_ctx *c, int slot);

@@ -259,6 +259,45 @@ class Genotyper:
         self._ck(self.L.vgb_call(self.h, _lib.ptr(g), _lib.ptr(c), self.n_sites))
         return g, c
 
+    # ---- output VCF ----
+    def vcf_template(self, vcf: bytes) -> None:
+        """vgb_vcf_template: the input SNP VCF (its bytes) as the output template of this context; needs the index"""
+        names = (C.c_char_p * len(self.chr_names))(*[n.encode() for n in self.chr_names])
+        lens = np.ascontiguousarray(self.chr_lens, dtype="<u8")
+        buf = np.frombuffer(vcf, dtype=np.uint8) if len(vcf) else np.zeros(1, np.uint8)
+        self._ck(self.L.vgb_vcf_template(self.h, _lib.ptr(buf), len(vcf), names, _lib.ptr(lens), len(self.chr_names)))
+
+    def vcf_template_copy(self, src: "Genotyper") -> None:
+        self._ck(self.L.vgb_vcf_template_copy(self.h, src.h))
+
+    @staticmethod
+    def _collector():
+        parts = []
+
+        def fn(user, p, n):
+            parts.append(C.string_at(p, n))
+            return 0
+        return parts, _lib.WRITE_FN(fn)
+
+    def vcf_write(self, gt: np.ndarray, gq: np.ndarray, bgzf: bool = False) -> bytes:
+        """vgb_vcf_write: this sample's VCF (BGZF with bgzf) from gtype and GQ per site (gq() of each called site's confidence)"""
+        gt = np.ascontiguousarray(gt, dtype=np.uint8)
+        gq = np.ascontiguousarray(gq, dtype="<i4")
+        assert gt.size == self.n_sites and gq.size == self.n_sites
+        parts, fn = self._collector()
+        self._ck(self.L.vgb_vcf_write(self.h, _lib.ptr(gt), _lib.ptr(gq), self.n_sites, int(bgzf), fn, None, None))
+        return b"".join(parts)
+
+    def deflate_bgzf(self, text, eof: bool = True) -> bytes:
+        """vgb_deflate_bgzf: BGZF members of host bytes, or of device memory given as (pointer, bytes)"""
+        parts, fn = self._collector()
+        if isinstance(text, tuple):
+            self._ck(self.L.vgb_deflate_bgzf(self.h, C.c_void_p(text[0]), text[1], 1, int(eof), fn, None))
+        else:
+            a = np.frombuffer(bytes(text), dtype=np.uint8) if len(text) else np.zeros(1, np.uint8)
+            self._ck(self.L.vgb_deflate_bgzf(self.h, _lib.ptr(a), len(text), 0, int(eof), fn, None))
+        return b"".join(parts)
+
     def counter_device_ptr(self) -> Tuple[int, int]:
         p, n = C.c_void_p(), C.c_uint64()
         self._ck(self.L.vgb_counter_device_ptr(self.h, C.byref(p), C.byref(n)))
@@ -351,3 +390,11 @@ def synth_genome_device(g: Genotyper, out_d: int, contig_starts, contig_lens, se
 def gq(conf: float) -> int:
     """(int)(-1*10*log(conf)), src/qv.cc:1681 -- CPython's math.log is the C library's log."""
     return int(-10.0 * math.log(conf))
+
+
+def site_gq(gt: np.ndarray, conf: np.ndarray) -> np.ndarray:
+    """GQ per site for vgb_vcf_write: gq() of every called site, 0 for the others"""
+    out = np.zeros(gt.size, dtype="<i4")
+    for i in np.flatnonzero(gt):
+        out[i] = gq(float(conf[i]))
+    return out
